@@ -10,6 +10,7 @@ energies (multistatesampler.py:776-782).  Strong scaling: the 256 replicas are s
   python bench.py --gpus 1 --steps 5 --warmup 3
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...        (the CPU arm: the oracle port of the reference's path, all host cores)
+  python bench.py ... --dump-outputs DIR      (also writes the arrays of the last timed iteration, to compare two builds)
 
 `value`   : device-resident loop (rx_run_iterations), CUDA events on the engine's stream, max over ranks.
 `e2e`     : the same iterations through the public API (ReplicaExchangeSampler.run with host_resident_states=True):
@@ -47,7 +48,13 @@ def parse():
                          "AlanineDipeptideVacuum (128 temperatures 300-600 K, 1000 steps/iteration; --replicas/--md-steps override)")
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-cpu-baseline', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed iteration computed (positions, velocities, '
+                         'energy matrix, replica -> state map, swap counts) as DIR/<name>.npy in float64')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -197,6 +204,42 @@ class Dist:
         return float(t[0])
 
 
+DUMP_LIMIT = 64 << 20      # bytes written by --dump-outputs at most
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each array as <path>/<name>.npy in float64 (the integer maps and counts are exact there).  Above
+    DUMP_LIMIT bytes in all, each array keeps a fixed, seeded sample of its rows and <name>_rows.npy lists them."""
+    arrays = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    with_rows = total + sum(8 * a.shape[0] for a in arrays.values() if a.ndim)     # each kept row costs 8 more bytes
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT and a.ndim and a.shape[0] > 1:
+            n = max(1, int(a.shape[0] * 0.9 * DUMP_LIMIT / with_rows))
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], n, replace=False))
+            np.save(os.path.join(path, name + '_rows.npy'), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(path, name + '.npy'), a)
+
+
+def engine_outputs(eng, dist):
+    """What the device-resident loop leaves for its caller after its last iteration; the replicas of every rank."""
+    def all_replicas(local):
+        full = np.zeros((eng.K,) + local.shape[1:])
+        full[eng.k0:eng.k1] = local
+        if dist.dist:
+            import torch
+            t = torch.from_numpy(full)
+            dist.dist.all_reduce(t, op=dist.dist.ReduceOp.SUM)
+            full = t.numpy()
+        return full
+    nacc, nprop = eng.get_mix_counts()
+    return {'positions': all_replicas(eng.get_positions()), 'velocities': all_replicas(eng.get_velocities()),
+            'energy_thermodynamic_states': eng.get_energies(), 'replica_thermodynamic_states': eng.get_replica_states(),
+            'n_accepted_matrix': nacc, 'n_proposed_matrix': nprop}
+
+
 # ------------------------------------------------------------------------------------------------------------
 def cpu_arm(args, steps, warmup, full_line):
     """The reference's CPU path restated (oracle/rx_oracle.c): numba-identical mixing (single thread, it is a
@@ -234,6 +277,10 @@ def cpu_arm(args, steps, warmup, full_line):
         t3 = time.time()
         if it >= warmup:
             times.append((t3 - t0, t1 - t0, t2 - t1, t3 - t2))
+    if full_line and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'positions': x, 'velocities': v, 'energy_thermodynamic_states': u,
+                                         'replica_thermodynamic_states': perm, 'n_accepted_matrix': nacc,
+                                         'n_proposed_matrix': nprop})
     tt = np.array(times)
     mean = tt[:, 0].mean()
     base = {'value': 1.0 / mean, 'unit': 'iterations/s', 'cores': threads, 'kind': 'port',
@@ -351,6 +398,10 @@ def cpu_arm_config4(args, steps, warmup, full_line):
         if it >= warmup:
             times.append((t3 - t0, t1 - t0, t2 - t1, t3 - t2))
     pool.shutdown()
+    if full_line and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'positions': np.stack(xs), 'velocities': np.stack(vs),
+                                         'energy_thermodynamic_states': u, 'replica_thermodynamic_states': perm,
+                                         'n_accepted_matrix': nacc, 'n_proposed_matrix': nprop})
     tt = np.array(times)
     mean = tt[:, 0].mean()
     base = {'value': 1.0 / mean, 'unit': 'iterations/s', 'cores': min(threads, K), 'kind': 'port',
@@ -406,6 +457,10 @@ def main_config4(args, world, rank):
     pt = eng.phase_times()
     mstats = eng.mix_stats()
     launches = dist.sum(pt['launches'])
+    if args.dump_outputs:
+        outputs = engine_outputs(eng, dist)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
     ms_iter = ms / args.steps
     peaks = {}
     try:
@@ -534,6 +589,10 @@ def main():
     pt = eng.phase_times()
     mstats = eng.mix_stats()
     launches = dist.sum(pt['launches'])
+    if args.dump_outputs:
+        outputs = engine_outputs(eng, dist)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
     value = args.steps / (ms * 1e-3)
 
     # roofline of k_propagate (the HBM-streaming kernel of SURVEY.md 8d): algorithmic bytes per launch

@@ -1,9 +1,11 @@
 #!/usr/bin/env python
 """Fixture for tests/test_openmm_adapter.py: the COMPLETE forces that the reference's AbsoluteAlchemicalFactory builds for
 the three configurations of make_alchemy_golden.py (every particle parameter, interaction group, global parameter, flag),
-serialised so that the GPU box -- which has no /root/reference -- can rebuild the stand-in objects and feed them to
-contrib.openmm_adapter.  Build container only.  Output: tests/golden/adapter_forces.json"""
-import json, os, sys
+serialised so that machines without the reference's source can rebuild the stand-in objects and feed them to
+contrib.openmm_adapter.  Needs the reference's source (make_alchemy_golden.load_factory).  Output:
+tests/golden/adapter_forces.json, and the SHA-256 of each configuration's forces as the reference factory built them in
+tests/golden/adapter_forces_sha256.json (what the test compares the fixture with)."""
+import hashlib, json, os, sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE); sys.path.insert(0, os.path.join(HERE, '..')); sys.path.insert(0, os.path.join(HERE, '..', '..'))
 import make_alchemy_golden as g
@@ -29,16 +31,22 @@ def dump(f):
     return d
 
 
+def digest(forces):
+    """SHA-256 of one configuration's dumped forces in canonical JSON."""
+    return hashlib.sha256(json.dumps(forces, sort_keys=True).encode()).hexdigest()
+
+
 if __name__ == '__main__':
     Factory, Region = g.load_factory()
     s = lj_setup(N=g.N, n_alch=g.N_ALCH, reduced_density=0.4, seed=77)
-    out = {}
+    out, sha = {}, {}
     for c, (annihilate, disable_lrc, (alpha, a, b, cc)) in enumerate(g.CONFIGS):
         factory = Factory(disable_alchemical_dispersion_correction=disable_lrc)
         region = Region(alchemical_atoms=list(range(g.N_ALCH)), annihilate_sterics=annihilate, softcore_alpha=alpha,
                         softcore_a=a, softcore_b=b, softcore_c=cc)
         forces = factory._alchemically_modify_NonbondedForce(g.reference_force(s), [region], frozenset())
         out['config%d' % c] = [dump(f) for v in forces.values() for f in v]
+        sha['config%d' % c] = digest(json.loads(json.dumps(out['config%d' % c])))
         # The same forces with a cutoff the engine (like OpenMM) accepts in this small box (r_c <= L/2): the energies the
         # GPU test compares with, again evaluated from the reference-emitted expressions inside the cutoff.
         U = []
@@ -58,3 +66,6 @@ if __name__ == '__main__':
     dst = os.path.join(HERE, 'adapter_forces.json')
     json.dump(out, open(dst, 'w'))
     print('wrote', dst, os.path.getsize(dst))
+    dst = os.path.join(HERE, 'adapter_forces_sha256.json')
+    json.dump(sha, open(dst, 'w'), indent=1)
+    print('wrote', dst)

@@ -1,14 +1,14 @@
 #!/usr/bin/env python
-"""Parameter fixture of testsystems.AlanineDipeptideVacuum: the reference's own input files
-(/root/reference/openmmtools/data/alanine-dipeptide-gbsa/alanine-dipeptide.{prmtop,crd}, read by
-testsystems.py:3375-3388) parsed by openmmtools_b200.amber and stored as plain numbers, so that the test system exists on
-machines without /root/reference.  Build container only.  Output: openmmtools_b200/data/alanine_dipeptide_vacuum.json"""
+"""Parameter fixture of testsystems.AlanineDipeptideVacuum: the original project's own input files for that test system
+(data/alanine-dipeptide-gbsa/alanine-dipeptide.{prmtop,crd}, read by testsystems.py:3375-3388; stored verbatim next to
+this script) parsed by openmmtools_b200.amber and stored as plain numbers, so that the package needs no AMBER files at
+run time.  Output: openmmtools_b200/data/alanine_dipeptide_vacuum.json"""
 import json, os, sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, '..', '..'))
 from openmmtools_b200 import amber
 
-SRC = '/root/reference/openmmtools/data/alanine-dipeptide-gbsa/alanine-dipeptide'
+SRC = os.path.join(HERE, 'alanine-dipeptide')
 
 
 def build():
