@@ -111,7 +111,7 @@ struct rx_engine {
     size_t ctile_cap = 0;
     unsigned char *d_filt = nullptr;   // 24-bit row image of u for the K=256 walker
     double *d_filt_scale = nullptr;    // [K] scales + [K] row abs-max
-    int prepared_kind = 0;        // ... with these records (REC_* of rx_mix.cu)
+    int prepared_plan = 0;        // walker plan (WalkPlan of rx_mix.cu) the prepared records were built for
     bool prepared = false;        // words + slot records for the next swap-all call were produced on stream_rng
     size_t last_consumed = 0;     // words the previous swap-all call consumed (sizes the generate-ahead)
     size_t slots_for_avail = 0;   // S.avail the slot records were built for

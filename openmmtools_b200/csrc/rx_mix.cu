@@ -16,6 +16,7 @@
 // in which no visited slot touches a replica swapped earlier in the same window is committed.
 #include "rx_internal.cuh"
 #include <type_traits>
+#include <algorithm>
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -221,16 +222,15 @@ __global__ void __launch_bounds__(256) k_slots_build(const uint32_t *__restrict_
 // (Round 1 had a producer warp and a ring synchronised by fences and volatile flags; the single warp with hardware-tracked
 // copies is racecheck-clean and costs ~6 more instructions per round.)
 //
-// Where the energies live (UMODE):
-//   U_FILTER24   the default for K <= 256 (at K = 256 the 512 KB of f64 do not fit; at smaller K the f32 filter is
-//                still faster than f64 comparisons): shared memory holds a 24-bit floating image of every row
-//                (delta = u - rowmin as a float32 truncated to sign + 8 exponent + 15 mantissa bits) that gives log_p
-//                to within a RIGOROUS bound eps = 3.2e-5 * sum|delta| + tiny; the decision is taken from the image, in
-//                f32, whenever it is more than eps away from both thresholds (log_p = 0 and log_p = log U); a round
-//                whose committed prefix contains an undecided lane is redone with the exact f64 values from L2.
-//                The result is therefore still bit-identical.
-//   U_F64_SMEM   the f64 matrix itself is in shared memory (K <= 128; RX_F64_SMEM=1 or RX_NO_FILTER=1)
-//   U_GLOBAL     exact f64 values from L2 every round (any larger K, or K = 256 with RX_NO_FILTER=1)
+// Where the energies live (FILTER):
+//   true    K <= 256, where the image fits in shared memory (213 KB at K = 256); the kernel finishes the passes of
+//           k_mix_walk2 on its SlotRec2 records.  Shared memory holds a 24-bit floating image of every row
+//           (delta = u - rowmin as a float32 truncated to sign + 8 exponent + 15 mantissa bits) that gives log_p
+//           to within a RIGOROUS bound eps = 3.2e-5 * sum|delta| + tiny; the decision is taken from the image, in
+//           f32, whenever it is more than eps away from both thresholds (log_p = 0 and log_p = log U); a round
+//           whose committed prefix contains an undecided lane is redone with the exact f64 values from L2.
+//           The result is therefore still bit-identical.
+//   false   exact f64 values from L2 every round, on SlotRec records (K >= 512)
 //
 // The walker's round is one dependent chain (~105 instructions, ~0.2 us); what was measured to matter, on one box:
 // no f64 on the chain (-65 ns), no data-dependent branch besides the loop's (-60 ns: one loop condition, predicated
@@ -240,31 +240,23 @@ __global__ void __launch_bounds__(256) k_slots_build(const uint32_t *__restrict_
 #define LOG_ACC_BIT 28
 #define LOG_STATE_BITS 14
 #define RING 1024
-enum { U_F64_SMEM = 0, U_FILTER24 = 1, U_GLOBAL = 2 };
 #include "rx_walk2.cuh"
-
-struct WalkShared {     // control words shared by the two warps
-    volatile unsigned prod;   // records [0, prod) of this pass are in the ring (modulo RING)
-    volatile unsigned head;   // walker position
-    volatile unsigned done;
-};
 #include "rx_walk_any.cuh"
 #include "rx_walk2c.cuh"
 
-// REC2: the records are SlotRec2 (rx_walk2.cuh); only with U_FILTER24, where this kernel finishes the passes of k_mix_walk2.
-template <int UMODE, bool REC2 = false>
+// FILTER: the records are SlotRec2 (rx_walk2.cuh), otherwise SlotRec.
+template <bool FILTER>
 __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict__ rec, const uint32_t *__restrict__ words,
                                                       unsigned nslots, const double *__restrict__ u, int K, int logK,
                                                       int *__restrict__ perm_g, uint32_t *__restrict__ commit_log,
                                                       const unsigned char *__restrict__ filt,
                                                       const double *__restrict__ filt_rowabs, MixCtl *ctl) {
     extern __shared__ double s_mix[];
-    // layout: ring[RING] 16-byte records | diag[K] f64 | (rowabs[K]) | (u f64 [K*K]) | perm[K] i32 | (image: u16[K*K] + u8[K*K])
+    // layout: ring[RING] 16-byte records | diag[K] f64 | (rowabs[K]) | perm[K] i32 | (image: u16[K*K] + u8[K*K])
     uint4 *s_ring = (uint4 *)s_mix;
     double *s_diag = s_mix + 2 * RING;
-    double *s_rowabs = s_diag + K;                                   // [K] |row minimum| (U_FILTER24 only)
-    double *s_u = s_rowabs + (UMODE == U_FILTER24 ? K : 0);
-    int *s_perm = (int *)(s_u + (UMODE == U_F64_SMEM ? (size_t)K * K : 0));
+    double *s_rowabs = s_diag + K;                                   // [K] |row minimum| (FILTER only)
+    int *s_perm = (int *)(s_rowabs + (FILTER ? K : 0));
     unsigned char *s_q = (unsigned char *)(s_perm + K);   // 24-bit image: int16 high plane [K*K] then uint8 low plane [K*K]
     // (the warp index through a shuffle: warp-uniform for the compiler, see k_mix_walk2)
     const int tid = threadIdx.x, lane = tid & 31, warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
@@ -273,11 +265,9 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
         s_perm[q] = st;
         s_diag[q] = u[((size_t)q << logK) + st];
         // per-row share of the f64-rounding bound, f32 rounded up: 1.6e-14 (|row minimum| + 1/2)
-        if (UMODE == U_FILTER24) ((float *)s_rowabs)[q] = __fmul_ru(1.6e-14f, __fadd_ru(__double2float_ru(filt_rowabs[q]), 0.5f));
+        if (FILTER) ((float *)s_rowabs)[q] = __fmul_ru(1.6e-14f, __fadd_ru(__double2float_ru(filt_rowabs[q]), 0.5f));
     }
-    if (UMODE == U_F64_SMEM)
-        for (int q = tid; q < K * K; q += 64) s_u[q] = u[q];
-    if (UMODE == U_FILTER24) {
+    if (FILTER) {
         const uint32_t *src = (const uint32_t *)filt;
         uint32_t *dst = (uint32_t *)s_q;
         for (int q = tid; q < (3 * K * K) / 4; q += 64) dst[q] = src[q];
@@ -328,7 +318,7 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
         const uint32_t ij = rq.x, backmask = rq.y;
         // the uniform an attempt here would draw belongs to the NEXT slot (SlotRec: its f64 logU is words z, w of the record)
         double logU_next = 0.0;
-        if (UMODE != U_FILTER24 || !REC2) {
+        if (!FILTER) {
             const uint2 lw = w2_lds64(ring_addr + (((w + 1) & (RING - 1)) << 4) + 8u);
             logU_next = __hiloint2double((int)lw.y, (int)lw.x);
         }
@@ -337,7 +327,7 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
         const unsigned a_ij = (i << logK) | (unsigned)sj, a_ji = (j << logK) | (unsigned)si;
         bool ge0, acc, undecided = false;
         double e_ij = 0.0, e_ji = 0.0;   // exact off-diagonal values, needed by the commit (new diagonal)
-        if (UMODE == U_FILTER24) {
+        if (FILTER) {
             // image of u: 24-bit floats of delta = u - rowmin; logp~ = (d_ii - d_ij) + (d_jj - d_ji), |logp~ - logp_ref| <= eps
             const unsigned a_ii = (i << logK) | (unsigned)si, a_jj = (j << logK) | (unsigned)sj;
             // (hi << 16) | (lo << 8) in one byte permute
@@ -355,7 +345,7 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
             const float eps = fmaf(mag, 3.2e-5f, (((const float *)s_rowabs)[i] + ((const float *)s_rowabs)[j]) + 1e-9f);
             // log of the uniform, rounded to f32 by the producer: |lu - logU| <= 2^-24 |lu|; d carries one more rounding
             // (SlotRec2: the f32 log-uniform of the next slot is the third word of this slot's own record)
-            const float lu = REC2 ? __uint_as_float(rq.z) : (float)logU_next;
+            const float lu = __uint_as_float(rq.z);
             const float d = lp - lu;
             const float mar = fmaf(fabsf(lp) + fabsf(lu), 1.3e-7f, eps);
             // |lp| > eps decides the sign of log_p, |d| > mar decides the comparison with the uniform (NaN: undecided)
@@ -367,8 +357,8 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
             const bool decided = ge0 || (dec_lp && dec_d);
             undecided = !decided;   // resolved below, and only if the lane turns out to matter
         } else {
-            e_ij = (UMODE == U_F64_SMEM) ? s_u[a_ij] : u[a_ij];
-            e_ji = (UMODE == U_F64_SMEM) ? s_u[a_ji] : u[a_ji];
+            e_ij = u[a_ij];
+            e_ji = u[a_ji];
             const double logp = swap_logp(e_ij, e_ji, s_diag[i], s_diag[j]);
             const double d = logp - logU_next;
             ge0 = logp >= 0.0;
@@ -407,7 +397,7 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
             // bit 32 (even position) of the skip word can only be set by the carry of an odd-start run
             advance = C ? (unsigned)__popc(low - 1u) : 32u + (sumO < X ? 1u : 0u);
         };
-        if (UMODE == U_FILTER24) {
+        if (FILTER) {
             // The filter's undecided lanes carry arbitrary ge0/acc.  Bits of V, C and cm below the lowest undecided
             // visited lane do not depend on them (the chain and the staleness test only look downwards), so the round
             // is resolved speculatively and redone with exact values only when such a lane lies inside the committed
@@ -421,7 +411,7 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
                     ge0 = logp >= 0.0;
                     acc = ge0;
                     if (!ge0) {
-                        const double dd = logp - (REC2 ? slot_logU(words, h + lane + 1) : rec[h + lane + 1].logU);
+                        const double dd = logp - slot_logU(words, h + lane + 1);
                         if (dd > 1e-9) acc = true;
                         else if (dd < -1e-9) acc = false;
                         else { const unsigned s1 = h + lane + 1; acc = mt_double(words[2 * (size_t)s1], words[2 * (size_t)s1 + 1]) < rx_exp_cr(logp); }
@@ -448,7 +438,7 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
         const bool swaps = mine && acc && i != j;  // an i == j lane must not write: a later committed lane may swap this replica
         if (mine) commit_log[log_at] = entry;
         if (swaps) { s_perm[i] = sj; s_perm[j] = si; }
-        if (UMODE != U_FILTER24) { if (swaps) { s_diag[i] = e_ij; s_diag[j] = e_ji; } }   // the image needs no f64 diagonal
+        if (!FILTER) { if (swaps) { s_diag[i] = e_ij; s_diag[j] = e_ji; } }   // the image needs no f64 diagonal
         logpos += n;
         h += advance;
         wpos = (wpos + advance) & (RING - 1);
@@ -480,7 +470,7 @@ __global__ void __launch_bounds__(64) k_mix_walk_pow2(const SlotRec *__restrict_
     }
 }
 
-// 24-bit row image of the energy matrix for the U_FILTER24 walker: delta = u[k,l] - min_l u[k,l] as a float32 truncated to
+// 24-bit row image of the energy matrix for the filter walkers: delta = u[k,l] - min_l u[k,l] as a float32 truncated to
 // its top 24 bits (sign, 8 exponent, 15 mantissa bits), stored as a uint16 plane followed by a uint8 plane.  Relative
 // precision 2^-15 per entry, so huge entries (a decoupled atom overlapping another one evaluated at lambda = 1) cost no
 // precision where the decisions are made.  absmax_out[k] = max |u[k,:]| (inf for rows with non-finite values).
@@ -738,27 +728,56 @@ struct MixTrace {   // RX_TRACE_MIX=1: device-time breakdown of one swap-all cal
 
 static inline bool is_pow2(int k) { return k >= 2 && (k & (k - 1)) == 0; }
 
-enum { REC_NONE = 0, REC_SLOT = 1, REC_SLOT2 = 2, REC_WORD = 3, REC_CAND = 4 };   // what prepare_pass builds from the stream
+// Which walkers run a swap-all call, a function of K alone:
+//   K                                 bulk of a pass          tail of a pass          records                counts from
+//   power of two, 2 .. 256            k_mix_walk2             k_mix_walk_pow2<true>   SlotRec2               k_mix_count_slots + k_mix_count
+//   power of two, 512 .. 16384        k_mix_walk_pow2<false>  (same kernel)           SlotRec                k_mix_count
+//   not a power of two, 3 .. 255      k_mix_walk2c            k_mix_walk_serial       SlotRec2 per candidate k_mix_count_slots
+//   not a power of two, 257 .. 4095   k_mix_walk_any          k_mix_walk_serial       WordRec                k_mix_count
+//   anything else                     k_mix_walk_serial
+// RX_WALK_SERIAL=1 gives every K that is not a power of two to the plain loop.
+enum WalkPlan { PLAN_SERIAL = 0, PLAN_FILTER, PLAN_L2, PLAN_CAND, PLAN_WORDS };
 
-static inline size_t pass_need(long long remaining, bool fast, bool anyk = false) {
+// Dynamic shared memory of every walker launch.  The walker is one latency-bound CTA: it claims (almost) a whole SM's shared
+// memory so that no other CTA -- in particular the stream generator that runs concurrently on the side stream -- is scheduled
+// onto the same SM and steals issue slots (226 KB + the walker's static shared memory + the generator's 8 KB exceed 228 KB).
+#define WALK_SMEM (226 * 1024)
+
+static int walk_plan(rx_engine *h, int K, WalkPlan *plan) {
+    if (is_pow2(K) && K <= (1 << LOG_STATE_BITS)) *plan = K <= 256 ? PLAN_FILTER : PLAN_L2;
+    else if (K >= 3 && K <= ANY_MAX_K && !getenv("RX_WALK_SERIAL")) *plan = K < 256 ? PLAN_CAND : PLAN_WORDS;
+    else *plan = PLAN_SERIAL;
+    size_t image_smem = 0;   // the layouts that hold the 24-bit row image (213 KB at K = 256)
+    if (*plan == PLAN_FILTER)   // k_mix_walk_pow2<true>: ring, diag, rowabs, perm, image; k_mix_walk2: ring, {state, diag}, image
+        image_smem = std::max((size_t)RING * 16 + (size_t)K * (2 * sizeof(double) + sizeof(int)) + (size_t)3 * K * K,
+                              (size_t)W2_RING * 16 + (size_t)K * sizeof(W2Replica) + (size_t)3 * K * K);
+    if (*plan == PLAN_CAND)     // k_mix_walk2c: ring, {state, diag}, image rows padded to an even length
+        image_smem = (size_t)W2_RING * 16 + (size_t)K * sizeof(W2Replica) + (size_t)((3 * K + 1) & ~1) * K;
+    if (image_smem > WALK_SMEM) RX_FAIL(h, RX_ERR_INVALID, "internal: the row image does not fit the walker's shared memory");
+    return RX_OK;
+}
+
+static inline size_t pass_need(long long remaining, WalkPlan plan) {
+    const bool anyk = plan == PLAN_CAND || plan == PLAN_WORDS;
     const size_t chunk_words = anyk ? (size_t)1 << 25 : (size_t)1 << 26;  // words per pass (any K: 16 bytes of records per word)
-    size_t need = fast ? (size_t)(4 * remaining + 160) : (size_t)(8 * remaining + 512);
+    const bool slots = plan == PLAN_FILTER || plan == PLAN_L2;
+    size_t need = slots ? (size_t)(4 * remaining + 160) : (size_t)(8 * remaining + 512);
     if (need > chunk_words) need = chunk_words;
     if (need < 512) need = 512;
     return need;
 }
 
-// Top the stream up to what a pass over `remaining` attempts may consume and (fast path) build its slot records,
-// on stream `st`.  Both are state independent, so for the NEXT mixing call this runs on the side stream while the
-// replicas are being propagated.
-static int prepare_pass(rx_engine *h, MTStream &S, long long remaining, bool fast, int kind, int K, cudaStream_t st, int *launches) {
-    const bool rec2 = kind == REC_SLOT2, candk = kind == REC_CAND, anyk = kind == REC_WORD || candk;
-    const size_t need = pass_need(remaining, fast, anyk);
+// Top the stream up to what a pass over `remaining` attempts may consume and build the plan's records from it, on stream
+// `st`.  Both are state independent, so for the NEXT mixing call this runs on the side stream while the replicas are
+// being propagated.
+static int prepare_pass(rx_engine *h, MTStream &S, long long remaining, WalkPlan plan, int K, cudaStream_t st, int *launches) {
+    const bool anyk = plan == PLAN_CAND || plan == PLAN_WORDS;   // records per word (candidate) rather than per slot
+    const size_t need = pass_need(remaining, plan);
     int rc = stream_reserve(h, S, 2 * need + 1024);   // room for the words generated ahead while the walker runs
     if (rc) return rc;
     rc = stream_fill(h, S, need, launches, st);
     if (rc) return rc;
-    if (fast || anyk) {
+    if (plan != PLAN_SERIAL) {
         const long long nslots = anyk ? (long long)S.avail : (long long)(S.avail / 2);   // records: per slot, or per word
         if ((size_t)nslots > h->slots_cap) {
             // size for the largest stream the buffer can ever hold (2 * need + 1024 words), so that the slightly different
@@ -777,7 +796,7 @@ static int prepare_pass(rx_engine *h, MTStream &S, long long remaining, bool fas
             RX_CHECK_CUDA(h, cudaMalloc(&h->d_slotlog, want * sizeof(uint32_t)));
             h->slots_cap = want;
         }
-        if (candk && (!h->d_cpos || h->ctile_cap < h->slots_cap)) {
+        if (plan == PLAN_CAND && (!h->d_cpos || h->ctile_cap < h->slots_cap)) {
             RX_CHECK_CUDA(h, cudaDeviceSynchronize());
             cudaFree(h->d_cpos); cudaFree(h->d_ctile);
             h->d_cpos = nullptr; h->d_ctile = nullptr;
@@ -785,7 +804,7 @@ static int prepare_pass(rx_engine *h, MTStream &S, long long remaining, bool fas
             RX_CHECK_CUDA(h, cudaMalloc(&h->d_ctile, (h->slots_cap / CAND_TILE + 8) * sizeof(uint32_t)));
             h->ctile_cap = h->slots_cap;
         }
-        if (candk) {
+        if (plan == PLAN_CAND) {
             // candidate coordinates (rx_walk2c.cuh): flag + count per tile, scan, scatter, one record per candidate index
             int nbits = 0;
             for (unsigned m = (unsigned)(K - 1); m; m >>= 1) nbits++;
@@ -797,12 +816,12 @@ static int prepare_pass(rx_engine *h, MTStream &S, long long remaining, bool fas
             k_cand_scatter<<<ntiles, 256, 0, st>>>(S.d_words, nslots, K, mask, h->d_ctile, h->d_cpos);
             k_cand_records<<<(unsigned)((nslots + 255) / 256), 256, 0, st>>>(S.d_words, h->d_cpos, d_ncand, mask, (SlotRec2 *)h->d_slots);
             *launches += 3;
-        } else if (anyk) {
+        } else if (plan == PLAN_WORDS) {
             static_assert(sizeof(WordRec) == sizeof(SlotRec), "all record formats share the d_slots buffer");
             int nbits = 0;
             for (unsigned m = (unsigned)(K - 1); m; m >>= 1) nbits++;
             k_words_build<<<(unsigned)((nslots + 255) / 256), 256, 0, st>>>(S.d_words, nslots, K, 0xffffffffu >> (32 - nbits), (WordRec *)h->d_slots);
-        } else if (rec2)
+        } else if (plan == PLAN_FILTER)
             k_slots_build2<<<(unsigned)((nslots + 255) / 256), 256, 0, st>>>(S.d_words, nslots, (uint32_t)(K - 1), (SlotRec2 *)h->d_slots);
         else
             k_slots_build<<<(unsigned)((nslots + 255) / 256), 256, 0, st>>>(S.d_words, nslots, (uint32_t)(K - 1), h->d_slots);
@@ -811,6 +830,25 @@ static int prepare_pass(rx_engine *h, MTStream &S, long long remaining, bool fas
     }
     h->slots_for_avail = S.avail;
     return RX_OK;
+}
+
+// Count matrices of a pass from a commit log: the sparse one indexed by slot or candidate (k_mix_walk2, k_mix_walk2c),
+// entries [0, n), or the dense one of k_mix_walk_pow2 and k_mix_walk_any, n entries.
+static int launch_count(rx_engine *h, bool sparse, long long n, int M, int *launches) {
+    if (n <= 0) return RX_OK;
+    long long nb = (n + 255) / 256;
+    if (nb > 148 * 16) nb = 148 * 16;
+    if (sparse) k_mix_count_slots<<<(unsigned)nb, 256, 0, h->stream>>>(h->d_slotlog, 0, n, M, h->d_nacc, h->d_nprop);
+    else k_mix_count<<<(unsigned)nb, 256, 0, h->stream>>>(h->d_log, n, M, h->d_nacc, h->d_nprop);
+    RX_CHECK_CUDA(h, cudaGetLastError());
+    (*launches)++;
+    return RX_OK;
+}
+
+// mix_stats[4]: device time of the walker launches between ev_walk[0] and ev_walk[1], in us (after a stream synchronise)
+static void add_walker_time(rx_engine *h) {
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, h->ev_walk[0], h->ev_walk[1]) == cudaSuccess) h->mix_stats[4] += (long long)(ms * 1e3f);
 }
 
 int rxi_mix_swap_all(rx_engine *h, long long nswap, int *launches) {
@@ -831,55 +869,24 @@ int rxi_mix_swap_all(rx_engine *h, long long nswap, int *launches) {
         RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream));
         return RX_OK;
     }
-    const bool fast = is_pow2(K) && K <= (1 << LOG_STATE_BITS);
-    // any other K up to 4095: the speculative walker over word positions (rx_walk_any.cuh); RX_WALK_SERIAL=1: the plain loop
-    const bool anyk = !fast && K >= 3 && K <= ANY_MAX_K && !getenv("RX_WALK_SERIAL");
+    WalkPlan plan;
+    int rc = walk_plan(h, K, &plan);
+    if (rc) return rc;
+    const bool pow2 = plan == PLAN_FILTER || plan == PLAN_L2;   // slot records; the walkers finish every pass themselves
     int logK = 0;
     while ((1 << logK) < K) logK++;
-    const size_t smem_small = (size_t)K * sizeof(int);
-    // ring (lu 8 + ij 4 + bm 4) + diag + perm
-    const size_t smem_base = (size_t)RING * 16 + (size_t)K * (sizeof(double) + sizeof(int));
-    const size_t smem_f64 = smem_base + (size_t)K * K * sizeof(double);
-    const size_t smem_f24 = smem_base + (size_t)K * sizeof(double) + (size_t)3 * K * K;
-    int umode = U_GLOBAL;
-    // the f32 row-image filter wherever it fits (K <= 256): it beats the f64 comparisons of U_F64_SMEM at every size
-    if (fast && smem_f24 <= 224 * 1024 && !getenv("RX_NO_FILTER") && !getenv("RX_F64_SMEM")) umode = U_FILTER24;
-    else if (fast && smem_f64 <= 200 * 1024) umode = U_F64_SMEM;
-    // filter mode: 16-byte SlotRec2 records, k_mix_walk2 for the bulk of a pass and k_mix_walk_pow2<U_FILTER24, true> for its tail
-    const bool rec2 = (umode == U_FILTER24);
-    const bool walk2 = rec2 && !getenv("RX_WALK_V1");
-    // any K <= 256 whose row image fits: the walker of k_mix_walk2 in candidate coordinates (rx_walk2c.cuh);
-    // RX_WALK_ANY_V1=1 keeps the word-position walker (cross-check)
-    const size_t smem_w2c = (size_t)W2_RING * 16 + (size_t)K * 8 + (size_t)((3 * K + 1) & ~1) * K;
-    const bool candk = anyk && K <= 256 && smem_w2c <= 224 * 1024 && !getenv("RX_WALK_ANY_V1") && !getenv("RX_NO_FILTER");
-    const int kind = candk ? REC_CAND : (anyk ? REC_WORD : (!fast ? REC_NONE : (rec2 ? REC_SLOT2 : REC_SLOT)));
-    const size_t smem_any_f64 = smem_base + (size_t)K * K * sizeof(double);
-    const bool any_smem = anyk && smem_any_f64 <= 200 * 1024;
-    const size_t smem_w2 = (size_t)W2_RING * 16 + (size_t)K * 8 + (size_t)3 * K * K;
-    size_t smem = !fast ? smem_small : (umode == U_F64_SMEM ? smem_f64 : (umode == U_FILTER24 ? smem_f24 : smem_base));
-    // The walker is one latency-bound CTA: claim (almost) a whole SM's shared memory so that no other CTA -- in particular
-    // the stream generator that runs concurrently on the side stream -- is scheduled onto the same SM and steals issue slots.
-    size_t smem_base_launch = smem_base;
-    if (fast) {
-        // 226 KB + this kernel's static shared memory + the generator's 8 KB exceed the SM's 228 KB
-        if (smem < 226 * 1024) smem = 226 * 1024;
-        smem_base_launch = 226 * 1024;
+    const size_t smem_serial = (size_t)K * sizeof(int);
+    if (smem_serial > 48 * 1024) RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk_serial, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_serial));
+    auto claim = [](const void *walker) { return cudaFuncSetAttribute(walker, cudaFuncAttributeMaxDynamicSharedMemorySize, WALK_SMEM); };
+    if (plan == PLAN_FILTER) {
+        RX_CHECK_CUDA(h, claim((const void *)k_mix_walk2));
+        RX_CHECK_CUDA(h, claim((const void *)k_mix_walk_pow2<true>));
     }
-    if (!fast) {
-        if (smem > 48 * 1024) RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk_serial, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        if (candk) RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk2c, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
-        if (anyk) {
-            RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk_any<U_F64_SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
-            RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk_any<U_GLOBAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
-        }
-    } else {
-        RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk_pow2<U_F64_SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk_pow2<U_FILTER24, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_mix_walk_pow2<U_GLOBAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_base_launch));
-    }
+    if (plan == PLAN_L2) RX_CHECK_CUDA(h, claim((const void *)k_mix_walk_pow2<false>));
+    if (plan == PLAN_CAND) RX_CHECK_CUDA(h, claim((const void *)k_mix_walk2c));
+    if (plan == PLAN_WORDS) RX_CHECK_CUDA(h, claim((const void *)k_mix_walk_any));
     tr.mark("func attributes");
-    if (umode == U_FILTER24 || candk) {
+    if (plan == PLAN_FILTER || plan == PLAN_CAND) {
         if (!h->d_filt) {
             RX_CHECK_CUDA(h, cudaMalloc(&h->d_filt, (size_t)3 * K * K + 16));
             RX_CHECK_CUDA(h, cudaMalloc(&h->d_filt_scale, sizeof(double) * 2 * K));
@@ -896,9 +903,8 @@ int rxi_mix_swap_all(rx_engine *h, long long nswap, int *launches) {
     const uint64_t consumed0 = S.consumed;
     const size_t chunk_words = (size_t)1 << 26;
     while (remaining > 0) {
-        const size_t need = pass_need(remaining, fast, anyk);
-        int rc;
-        if (h->prepared && h->prepared_kind == kind && S.avail >= need && h->slots_for_avail == S.avail) {
+        const size_t need = pass_need(remaining, plan);
+        if (h->prepared && h->prepared_plan == plan && S.avail >= need && h->slots_for_avail == S.avail) {
             // produced on the side stream while the replicas were propagating
             RX_CHECK_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_prepared, 0));
             float ms = 0;
@@ -908,7 +914,7 @@ int rxi_mix_swap_all(rx_engine *h, long long nswap, int *launches) {
             h->mix_stats[5] += (long long)(rx_wall_us() - tw0);
         } else {
             if (h->prepared) RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream_rng));
-            rc = prepare_pass(h, S, remaining, fast, kind, K, h->stream, launches);
+            rc = prepare_pass(h, S, remaining, plan, K, h->stream, launches);
             if (rc) return rc;
         }
         h->prepared = false;
@@ -916,7 +922,7 @@ int rxi_mix_swap_all(rx_engine *h, long long nswap, int *launches) {
         MixCtl ctl = {0, remaining, 0, 0, 0, 0, 0};
         RX_CHECK_CUDA(h, cudaMemcpyAsync(h->d_ctl, &ctl, sizeof(ctl), cudaMemcpyHostToDevice, h->stream));
         size_t consumed_words;
-        if (fast) {
+        if (pow2) {
             const long long nslots = (long long)(S.avail / 2);
             // While the walker runs (it only reads words [0, avail)), generate on the side stream about as many words
             // as the previous call consumed: they are appended behind the valid region and adopted afterwards.
@@ -929,96 +935,62 @@ int rxi_mix_swap_all(rx_engine *h, long long nswap, int *launches) {
                 *launches += 1;
             }
             RX_CHECK_CUDA(h, cudaEventRecord(h->ev_walk[0], h->stream));
-            if (umode == U_F64_SMEM)
-                k_mix_walk_pow2<U_F64_SMEM><<<1, 64, smem, h->stream>>>(h->d_slots, S.d_words, (unsigned)nslots, h->d_u, K, logK, h->d_perm, h->d_log, nullptr, nullptr, h->d_ctl);
-            else if (umode == U_FILTER24) {
-                if (walk2) {
-                    static_assert(sizeof(SlotRec2) == sizeof(SlotRec), "both record formats share the d_slots buffer");
-                    if (smem_w2 > smem) RX_FAIL(h, RX_ERR_INVALID, "internal: k_mix_walk2 shared memory");
-                    // sparse commit log: one word per slot, zero = no attempt started there
-                    RX_CHECK_CUDA(h, cudaMemsetAsync(h->d_slotlog, 0, (size_t)nslots * sizeof(uint32_t), h->stream));
-                    k_mix_walk2<<<1, W2_THREADS, smem, h->stream>>>((const SlotRec2 *)h->d_slots, S.d_words, (unsigned)nslots, h->d_u, K, logK, h->d_perm, h->d_slotlog, h->d_filt, h->d_filt_scale, h->d_ctl);
-                    RX_CHECK_CUDA(h, cudaGetLastError());
-                    *launches += 1;
-                }
-                k_mix_walk_pow2<U_FILTER24, true><<<1, 64, smem, h->stream>>>(h->d_slots, S.d_words, (unsigned)nslots, h->d_u, K, logK, h->d_perm, h->d_log, h->d_filt, h->d_filt_scale, h->d_ctl);
-            }
-            else
-                k_mix_walk_pow2<U_GLOBAL><<<1, 64, smem_base_launch, h->stream>>>(h->d_slots, S.d_words, (unsigned)nslots, h->d_u, K, logK, h->d_perm, h->d_log, nullptr, nullptr, h->d_ctl);
+            if (plan == PLAN_FILTER) {
+                static_assert(sizeof(SlotRec2) == sizeof(SlotRec), "both record formats share the d_slots buffer");
+                // sparse commit log: one word per slot, zero = no attempt started there
+                RX_CHECK_CUDA(h, cudaMemsetAsync(h->d_slotlog, 0, (size_t)nslots * sizeof(uint32_t), h->stream));
+                k_mix_walk2<<<1, W2_THREADS, WALK_SMEM, h->stream>>>((const SlotRec2 *)h->d_slots, S.d_words, (unsigned)nslots, h->d_u, K, logK, h->d_perm, h->d_slotlog, h->d_filt, h->d_filt_scale, h->d_ctl);
+                RX_CHECK_CUDA(h, cudaGetLastError());
+                *launches += 1;
+                k_mix_walk_pow2<true><<<1, 64, WALK_SMEM, h->stream>>>(h->d_slots, S.d_words, (unsigned)nslots, h->d_u, K, logK, h->d_perm, h->d_log, h->d_filt, h->d_filt_scale, h->d_ctl);
+            } else
+                k_mix_walk_pow2<false><<<1, 64, WALK_SMEM, h->stream>>>(h->d_slots, S.d_words, (unsigned)nslots, h->d_u, K, logK, h->d_perm, h->d_log, nullptr, nullptr, h->d_ctl);
             RX_CHECK_CUDA(h, cudaGetLastError());
             RX_CHECK_CUDA(h, cudaEventRecord(h->ev_walk[1], h->stream));
             tr.mark("walker");
             *launches += 1;
             RX_CHECK_CUDA(h, cudaMemcpyAsync(&ctl, h->d_ctl, sizeof(ctl), cudaMemcpyDeviceToHost, h->stream));
             RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream));
-            { float wms = 0; if (cudaEventElapsedTime(&wms, h->ev_walk[0], h->ev_walk[1]) == cudaSuccess) h->mix_stats[4] += (long long)(wms * 1e3f); }
+            add_walker_time(h);
             consumed_words = (size_t)(2 * ctl.head);
             if (ahead) {   // adopt the words generated during the walk
                 RX_CHECK_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_prepared, 0));
                 S.avail += ahead;
             }
-            if (walk2 && ctl.head > 0) {
-                long long nb = (ctl.head + 255) / 256;
-                if (nb > 148 * 16) nb = 148 * 16;
-                k_mix_count_slots<<<(unsigned)nb, 256, 0, h->stream>>>(h->d_slotlog, 0, ctl.head, M, h->d_nacc, h->d_nprop);
-                RX_CHECK_CUDA(h, cudaGetLastError());
-                *launches += 1;
+            if (plan == PLAN_FILTER) {   // k_mix_walk2 logs by slot, up to the one it reached
+                rc = launch_count(h, true, ctl.head, M, launches);
+                if (rc) return rc;
             }
-            if (ctl.log_count > 0) {
-                long long nb = (ctl.log_count + 255) / 256;
-                if (nb > 148 * 16) nb = 148 * 16;
-                k_mix_count<<<(unsigned)nb, 256, 0, h->stream>>>(h->d_log, ctl.log_count, M, h->d_nacc, h->d_nprop);
-                RX_CHECK_CUDA(h, cudaGetLastError());
-                *launches += 1;
-            }
+            rc = launch_count(h, false, ctl.log_count, M, launches);
+            if (rc) return rc;
             tr.mark("adopt-ahead + count");
         } else {
-            if (candk) {
-                // bulk of the pass: the walk2 organisation over candidate indices; the plain loop below finishes the pass
+            if (plan != PLAN_SERIAL) {
+                // bulk of the pass; what the walker leaves -- the last words of the pass -- is finished by the plain loop below
                 RX_CHECK_CUDA(h, cudaEventRecord(h->ev_walk[0], h->stream));
-                RX_CHECK_CUDA(h, cudaMemsetAsync(h->d_slotlog, 0, S.avail * sizeof(uint32_t), h->stream));
-                k_mix_walk2c<<<1, W2_THREADS, 226 * 1024, h->stream>>>((const SlotRec2 *)h->d_slots, S.d_words, h->d_cpos,
-                                                                        h->d_ctile + (h->ctile_cap / CAND_TILE + 4), h->d_u, K, h->d_perm,
-                                                                        h->d_slotlog, h->d_filt, h->d_filt_scale, h->d_ctl);
-                RX_CHECK_CUDA(h, cudaGetLastError());
-                RX_CHECK_CUDA(h, cudaEventRecord(h->ev_walk[1], h->stream));
-                *launches += 1;
-            } else if (anyk) {
-                // bulk of the pass: speculative walker over word positions (claims the SM like the power-of-two walkers);
-                // what it leaves -- the last words of the pass -- is finished by the plain loop below
-                RX_CHECK_CUDA(h, cudaEventRecord(h->ev_walk[0], h->stream));
-                if (any_smem)
-                    k_mix_walk_any<U_F64_SMEM><<<1, 64, 226 * 1024, h->stream>>>((const WordRec *)h->d_slots, S.d_words, (unsigned)S.avail, h->d_u, K, h->d_perm, h->d_log, h->d_ctl);
-                else
-                    k_mix_walk_any<U_GLOBAL><<<1, 64, 226 * 1024, h->stream>>>((const WordRec *)h->d_slots, S.d_words, (unsigned)S.avail, h->d_u, K, h->d_perm, h->d_log, h->d_ctl);
+                if (plan == PLAN_CAND) {
+                    RX_CHECK_CUDA(h, cudaMemsetAsync(h->d_slotlog, 0, S.avail * sizeof(uint32_t), h->stream));
+                    k_mix_walk2c<<<1, W2_THREADS, WALK_SMEM, h->stream>>>((const SlotRec2 *)h->d_slots, S.d_words, h->d_cpos,
+                                                                          h->d_ctile + (h->ctile_cap / CAND_TILE + 4), h->d_u, K, h->d_perm,
+                                                                          h->d_slotlog, h->d_filt, h->d_filt_scale, h->d_ctl);
+                } else
+                    k_mix_walk_any<<<1, 64, WALK_SMEM, h->stream>>>((const WordRec *)h->d_slots, S.d_words, (unsigned)S.avail, h->d_u, K, h->d_perm, h->d_log, h->d_ctl);
                 RX_CHECK_CUDA(h, cudaGetLastError());
                 RX_CHECK_CUDA(h, cudaEventRecord(h->ev_walk[1], h->stream));
                 *launches += 1;
             }
-            k_mix_walk_serial<<<1, 32, smem, h->stream>>>(S.d_words, (long long)S.avail, h->d_u, K, M, h->d_perm, h->d_nacc,
-                                                        h->d_nprop, h->d_ctl);
+            k_mix_walk_serial<<<1, 32, smem_serial, h->stream>>>(S.d_words, (long long)S.avail, h->d_u, K, M, h->d_perm, h->d_nacc,
+                                                               h->d_nprop, h->d_ctl);
             RX_CHECK_CUDA(h, cudaGetLastError());
             *launches += 1;
             RX_CHECK_CUDA(h, cudaMemcpyAsync(&ctl, h->d_ctl, sizeof(ctl), cudaMemcpyDeviceToHost, h->stream));
             RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream));
             consumed_words = (size_t)ctl.head;
-            if (anyk) {
-                float wms = 0;
-                if (cudaEventElapsedTime(&wms, h->ev_walk[0], h->ev_walk[1]) == cudaSuccess) h->mix_stats[4] += (long long)(wms * 1e3f);
-                if (candk && ctl.aux > 0) {
-                    long long nb = (ctl.aux + 255) / 256;
-                    if (nb > 148 * 16) nb = 148 * 16;
-                    k_mix_count_slots<<<(unsigned)nb, 256, 0, h->stream>>>(h->d_slotlog, 0, ctl.aux, M, h->d_nacc, h->d_nprop);
-                    RX_CHECK_CUDA(h, cudaGetLastError());
-                    *launches += 1;
-                }
-                if (!candk && ctl.log_count > 0) {
-                    long long nb = (ctl.log_count + 255) / 256;
-                    if (nb > 148 * 16) nb = 148 * 16;
-                    k_mix_count<<<(unsigned)nb, 256, 0, h->stream>>>(h->d_log, ctl.log_count, M, h->d_nacc, h->d_nprop);
-                    RX_CHECK_CUDA(h, cudaGetLastError());
-                    *launches += 1;
-                }
+            if (plan != PLAN_SERIAL) {
+                add_walker_time(h);
+                // k_mix_walk2c logs by candidate index, up to the one it reached
+                rc = plan == PLAN_CAND ? launch_count(h, true, ctl.aux, M, launches) : launch_count(h, false, ctl.log_count, M, launches);
+                if (rc) return rc;
             }
         }
         if (ctl.remaining == remaining && consumed_words == 0 && need >= chunk_words)
@@ -1040,8 +1012,8 @@ int rxi_mix_swap_all(rx_engine *h, long long nswap, int *launches) {
         RX_CHECK_CUDA(h, cudaStreamWaitEvent(h->stream_rng, h->ev_consumed, 0));
         RX_CHECK_CUDA(h, cudaEventRecord(h->ev[6], h->stream_rng));
         int l2 = 0;
-        int rc2 = prepare_pass(h, S, nswap, fast, kind, K, h->stream_rng, &l2);
-        h->prepared_kind = kind;
+        int rc2 = prepare_pass(h, S, nswap, plan, K, h->stream_rng, &l2);
+        h->prepared_plan = plan;
         if (rc2) return rc2;
         RX_CHECK_CUDA(h, cudaEventRecord(h->ev[7], h->stream_rng));
         RX_CHECK_CUDA(h, cudaEventRecord(h->ev_prepared, h->stream_rng));

@@ -1,6 +1,6 @@
 // rx_walk2.cuh -- second-generation swap-all walker for power-of-two K <= 256 (included by rx_mix.cu).
 //
-// Same algorithm and the same results as k_mix_walk_pow2<U_FILTER24> (replicaexchange.py:321-349 bit for bit); what
+// Same algorithm and the same results as k_mix_walk_pow2<true> (replicaexchange.py:321-349 bit for bit); what
 // changes is the length of the dependent chain of one speculation round:
 //   * lane <-> slot mapping is FIXED (lane = slot mod 32) and the window [h, h+32) rotates over the lanes, so a lane
 //     keeps its slot record in registers until the slot leaves the window and the record of its next slot (s + 32)
@@ -13,7 +13,7 @@
 //   * a second warp turns the records into ready-to-use slot contexts in a shared-memory ring (release/acquire fence
 //     patterns on its two control words): the walker's round is bound by its instruction count, not by latency.
 // The kernel runs the bulk of a pass; the last < 600 slots / < 130 attempts of a pass are left to
-// k_mix_walk_pow2<U_FILTER24, true>, which reads the same records.
+// k_mix_walk_pow2<true>, which reads the same records.
 #pragma once
 
 struct SlotRec2 {        // 16 bytes, one 2-word slot of the stream, state independent
@@ -74,7 +74,7 @@ __global__ void __launch_bounds__(256) k_slots_build2(const uint32_t *__restrict
 }
 
 // The filter's decision for one (i, j, si, sj): image values d_x = image of u[x, s_x] - rowmin_x (the maintained diagonal)
-// and f_xy = image of u[x, s_y] - rowmin_x.  Same rigorous bound as k_mix_walk_pow2<U_FILTER24> (see its derivation there;
+// and f_xy = image of u[x, s_y] - rowmin_x.  Same rigorous bound as k_mix_walk_pow2<true> (see its derivation there;
 // the factor 3.2e-5 leaves 5 % over the 2^-15 + 2^-23 the roundings need, far more than the re-association below costs):
 //   e0  = 3.2e-5 (|d_i| + |d_j|) + eps0        as soon as the states are known (before the image loads return),
 //   eps = 3.2e-5 (|f_ij| + |f_ji|) + e0,       lp = (d_i - f_ij) + (d_j - f_ji),

@@ -75,19 +75,23 @@ __global__ void __launch_bounds__(256) k_words_build(const uint32_t *__restrict_
     rec[p] = r;
 }
 
+struct WalkShared {     // control words shared by the two warps
+    volatile unsigned prod;   // records [0, prod) of this pass are in the ring (modulo RING)
+    volatile unsigned head;   // walker position
+    volatile unsigned done;
+};
+
 // CTA = 2 warps, organised like k_mix_walk_pow2: warp 1 streams the records into a shared-memory ring, warp 0 walks.
-// head counts WORDS.  UMODE: U_F64_SMEM (the f64 matrix in shared memory) or U_GLOBAL (from L2).
-template <int UMODE>
+// head counts WORDS.  The energies are read from L2.
 __global__ void __launch_bounds__(64) k_mix_walk_any(const WordRec *__restrict__ rec, const uint32_t *__restrict__ words,
                                                      unsigned nwords, const double *__restrict__ u, int K,
                                                      int *__restrict__ perm_g, uint32_t *__restrict__ commit_log, MixCtl *ctl) {
     extern __shared__ double s_mix[];
     __shared__ WalkShared sh;
-    // layout: ring_lu[RING] f64 | diag[K] f64 | (u f64 [K*K]) | ring_ijl[RING] u32 | ring_bm[RING] u32 | perm[K] i32
+    // layout: ring_lu[RING] f64 | diag[K] f64 | ring_ijl[RING] u32 | ring_bm[RING] u32 | perm[K] i32
     double *ring_lu = s_mix;
     double *s_diag = ring_lu + RING;
-    double *s_u = s_diag + K;
-    uint32_t *ring_ijl = (uint32_t *)(s_u + (UMODE == U_F64_SMEM ? (size_t)K * K : 0));
+    uint32_t *ring_ijl = (uint32_t *)(s_diag + K);
     uint32_t *ring_bm = ring_ijl + RING;
     int *s_perm = (int *)(ring_bm + RING);
     // (the warp index through a shuffle: warp-uniform for the compiler, see k_mix_walk2)
@@ -97,8 +101,6 @@ __global__ void __launch_bounds__(64) k_mix_walk_any(const WordRec *__restrict__
         s_perm[q] = st;
         s_diag[q] = u[(size_t)q * K + st];
     }
-    if (UMODE == U_F64_SMEM)
-        for (int q = tid; q < K * K; q += 64) s_u[q] = u[q];
     const unsigned head0 = (unsigned)ctl->head;
     if (tid == 0) { sh.prod = head0; sh.head = head0; sh.done = 0; }
     __syncthreads();
@@ -164,8 +166,8 @@ __global__ void __launch_bounds__(64) k_mix_walk_any(const WordRec *__restrict__
         const bool unknown = len == 0u;
         const int si = s_perm[i], sj = s_perm[j];
         const unsigned a_ij = i * (unsigned)K + (unsigned)sj, a_ji = j * (unsigned)K + (unsigned)si;
-        const double e_ij = (UMODE == U_F64_SMEM) ? s_u[a_ij] : u[a_ij];
-        const double e_ji = (UMODE == U_F64_SMEM) ? s_u[a_ji] : u[a_ji];
+        const double e_ij = u[a_ij];
+        const double e_ji = u[a_ji];
         const double logp = swap_logp(e_ij, e_ji, s_diag[i], s_diag[j]);
         const double d = logp - lu;
         const bool ge0 = logp >= 0.0;

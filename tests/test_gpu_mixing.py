@@ -88,20 +88,20 @@ def test_swap_all_full_size_vs_oracle(K, model, seed):
 @pytest.mark.parametrize('K,model,nswap,seed', [(3, 'flat', 200_000, 31), (5, 'normal', 200_000, 32), (12, 'flat', 300_000, 33),
                                                 (65, 'flat', 65 ** 3, 34), (100, 'normal', 100 ** 3, 35),
                                                 (127, 'ladder', 500_000, 36), (129, 'normal', 500_000, 37),
-                                                (200, 'normal', 2_000_000, 38), (1000, 'flat', 1_000_000, 39)])
-@pytest.mark.parametrize('path', ['default', 'serial', 'words'])
+                                                (200, 'normal', 2_000_000, 38), (257, 'normal', 300_000, 40),
+                                                (300, 'flat', 300_000, 41), (383, 'ladder', 300_000, 42),
+                                                (600, 'ladder', 1_000_000, 43), (767, 'normal', 300_000, 44),
+                                                (1000, 'flat', 1_000_000, 39), (2047, 'normal', 300_000, 45)])
+@pytest.mark.parametrize('path', ['default', 'serial'])
 def test_swap_all_any_k_vs_oracle(monkeypatch, K, model, nswap, seed, path):
-    """K that is not a power of two.  default: the walk2 organisation in candidate coordinates (k_mix_walk2c, K <= 256) or the
-    walker over word positions (k_mix_walk_any: above 256, or everywhere with RX_WALK_ANY_V1=1 -- the f64 matrix in shared
-    memory up to K ~ 150, from L2 above); with RX_WALK_SERIAL=1 the plain loop; three iterations each."""
+    """K that is not a power of two.  default: the walk2 organisation in candidate coordinates (k_mix_walk2c, K < 256) or the
+    walker over word positions (k_mix_walk_any, 257 <= K <= 4095), each followed by the plain loop for the end of a pass;
+    with RX_WALK_SERIAL=1 the plain loop alone; three iterations each."""
     from oracle import oracle
     serial = path == 'serial'
     if serial:
         if nswap > 300_000: pytest.skip('the plain loop takes 0.6 us per attempt')
         monkeypatch.setenv('RX_WALK_SERIAL', '1')
-    if path == 'words':
-        if K > 256: pytest.skip('already the default above K = 256')
-        monkeypatch.setenv('RX_WALK_ANY_V1', '1')
     u = energies(model, K, 777 + K)
     e = gpu_engine(0, K, K)
     e.set_energies(u)
@@ -131,7 +131,8 @@ def test_swap_all_any_k_vs_oracle(monkeypatch, K, model, nswap, seed, path):
     e.close()
 
 
-@pytest.mark.parametrize('K,kind', [(100, 'equal_rows'), (100, 'nonfinite'), (37, 'equal_rows')])
+@pytest.mark.parametrize('K,kind', [(100, 'equal_rows'), (100, 'nonfinite'), (37, 'equal_rows'), (300, 'equal_rows'),
+                                    (300, 'nonfinite')])
 def test_swap_all_any_k_hard_matrices(K, kind):
     """Identical rows (iteration 0 of a run whose replicas start from one configuration: every log_p is a rounding error
     around 0) and non-finite entries."""
@@ -289,13 +290,11 @@ def test_swap_all_with_nonfinite_and_huge_energies(K):
         e.close()
 
 
-@pytest.mark.parametrize('env,K,model', [('RX_F64_SMEM', 16, 'flat'), ('RX_F64_SMEM', 64, 'normal'), ('RX_F64_SMEM', 128, 'flat'),
-                                         ('RX_NO_FILTER', 64, 'flat'), ('RX_NO_FILTER', 256, 'flat')])
-def test_swap_all_other_energy_placements_vs_oracle(monkeypatch, env, K, model):
-    """The walker variants the default selection no longer reaches: the f64 matrix in shared memory (RX_F64_SMEM /
-    RX_NO_FILTER at K <= 128) and the exact values from L2 every round (RX_NO_FILTER at K = 256)."""
+@pytest.mark.parametrize('K,model', [(16, 'flat'), (64, 'normal'), (128, 'flat'), (256, 'flat'), (1024, 'flat')])
+def test_swap_all_pow2_walkers_vs_oracle(K, model):
+    """Both power-of-two walkers at up to 1.5 M attempts per call: the row-image filter (k_mix_walk2 and k_mix_walk_pow2<true>,
+    K <= 256) and the exact values from L2 every round (k_mix_walk_pow2<false>, K >= 512)."""
     from oracle import oracle
-    monkeypatch.setenv(env, '1')
     u = energies(model, K, 977 + K)
     e = gpu_engine(0, K, K)
     e.set_energies(u)
@@ -308,6 +307,6 @@ def test_swap_all_other_energy_placements_vs_oracle(monkeypatch, env, K, model):
         st, nacc, nprop = e.mix_swap_all(nswap)
         na = np.zeros((K, K), np.int64); npr = np.zeros((K, K), np.int64)
         oracle.mix_swap_all(mt, nswap, st_o, u, na, npr)
-        assert np.array_equal(st, st_o), (env, K, it)
+        assert np.array_equal(st, st_o), (K, it)
         assert np.array_equal(nacc, na) and np.array_equal(nprop, npr)
     e.close()

@@ -1,7 +1,7 @@
 """A/B timing of the swap-all walker builds on one GPU (development aid).
   python tools/ab_walk.py libA.so libB.so ...     each library runs in its own process (RX_B200_LIB), K = 256 on the
   real alchemical-LJ energy matrix tools/data/u_lj_256.npy; prints walker ms, rounds, ns/round and a permutation digest
-  (all builds must print the same digest).  'v1' as a library name = the default library with RX_WALK_V1=1."""
+  (all builds must print the same digest)."""
 import os, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -25,10 +25,7 @@ print('walker %%8.2f ms (best of %%d)  rounds %%d  %%6.1f ns/round  digests %%s'
 
 for lib in sys.argv[1:]:
     env = dict(os.environ)
-    if lib == 'v1':
-        env['RX_WALK_V1'] = '1'
-        env.pop('RX_B200_LIB', None)
-    elif lib != 'default':
+    if lib != 'default':
         env['RX_B200_LIB'] = os.path.abspath(lib)
     try:
         r = subprocess.run([sys.executable, '-c', CHILD], env=env, capture_output=True, text=True, timeout=int(os.environ.get('AB_TIMEOUT', '90')))

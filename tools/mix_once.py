@@ -1,5 +1,6 @@
-"""One swap-all call (for ncu captures of the walkers): the K=256 LJ energy matrix, or with K given, a K x K sub-matrix of it
-(any K <= 256: k_mix_walk_any for K not a power of two).  usage: mix_once.py [nswap [K]]"""
+"""One swap-all call (for ncu captures of the walkers): the K=256 LJ energy matrix, or with K given, a K x K matrix sampled
+from its rows and columns (rows repeat above K = 256); K not a power of two runs k_mix_walk2c below 256 and k_mix_walk_any
+above.  usage: mix_once.py [nswap [K]]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
