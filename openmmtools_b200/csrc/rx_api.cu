@@ -3,9 +3,7 @@
 #include "rx_internal.cuh"
 #include <dlfcn.h>
 #include <math.h>
-#include <stdio.h>
 #include <string.h>
-#include <stdlib.h>
 
 thread_local std::string g_rx_create_error;
 
@@ -50,6 +48,7 @@ extern "C" int rx_create(const rx_config *cfg, rx_engine **out) {
     CREATE_CUDA(cudaSetDevice(cfg->device));
     h = new rx_engine();
     h->cfg = *cfg;
+    CREATE_CUDA(cudaDeviceGetAttribute(&h->n_sms, cudaDevAttrMultiProcessorCount, cfg->device));
     const int K = cfg->n_replicas, M = cfg->n_states, N = cfg->n_atoms, W = cfg->world_size, R = cfg->rank;
     h->k0 = (int)(((long long)R * K) / W);
     h->kloc = (int)(((long long)(R + 1) * K) / W) - h->k0;
@@ -220,23 +219,33 @@ extern "C" int rx_set_states(rx_engine *h, const rx_state_params *s) {
     return RX_OK;
 }
 
-extern "C" int rx_set_integrator(rx_engine *h, double timestep, double collision_rate, int32_t n_steps,
-                                 const char *splitting) {
-    ENTER(h);
-    if (!(timestep > 0) || collision_rate < 0 || n_steps < 0) RX_FAIL(h, RX_ERR_INVALID, "rx_set_integrator: bad timestep/collision_rate/n_steps");
-    if (!splitting) RX_FAIL(h, RX_ERR_INVALID, "rx_set_integrator: null splitting");
+// Checks the arguments of a move (messages start with `who`) and stores it in *out; *out is untouched on failure.
+static int make_move(rx_engine *h, const char *who, double timestep, double collision_rate, int32_t n_steps,
+                     const char *splitting, int reassign, rx_state_move *out) {
+    const std::string w(who);
+    if (!(timestep > 0) || collision_rate < 0 || n_steps < 0) RX_FAIL(h, RX_ERR_INVALID, w + ": bad timestep/collision_rate/n_steps");
+    if (!splitting) RX_FAIL(h, RX_ERR_INVALID, w + ": null splitting");
     const size_t n = strlen(splitting);
-    if (n == 0 || n >= RX_MAX_PROGRAM) RX_FAIL(h, RX_ERR_INVALID, "rx_set_integrator: splitting must have 1..31 substeps");
+    if (n == 0 || n >= RX_MAX_PROGRAM) RX_FAIL(h, RX_ERR_INVALID, w + ": splitting must have 1..31 substeps");
     bool hasV = false, hasR = false, hasO = false;
     for (size_t i = 0; i < n; i++) {
         const char c = splitting[i];
         if (c == 'V') hasV = true; else if (c == 'R') hasR = true; else if (c == 'O') hasO = true;
-        else RX_FAIL(h, RX_ERR_UNSUPPORTED, "rx_set_integrator: only R, V and O substeps are supported (no force groups / Metropolization)");
+        else RX_FAIL(h, RX_ERR_UNSUPPORTED, w + ": only R, V and O substeps are supported (no force groups / Metropolization)");
     }
-    if (!(hasV && hasR && hasO)) RX_FAIL(h, RX_ERR_INVALID, "rx_set_integrator: splitting must contain R, V and O (integrators.py:1360-1363)");
-    h->dt = timestep; h->gamma = collision_rate; h->n_steps = n_steps;
-    memset(h->program, 0, sizeof(h->program));
-    memcpy(h->program, splitting, n);
+    if (!(hasV && hasR && hasO)) RX_FAIL(h, RX_ERR_INVALID, w + ": splitting must contain R, V and O (integrators.py:1360-1363)");
+    rx_state_move m;
+    m.dt = timestep; m.gamma = collision_rate; m.n_steps = n_steps; m.reassign = reassign ? 1 : 0;
+    memcpy(m.program, splitting, n);
+    *out = m;
+    return RX_OK;
+}
+
+extern "C" int rx_set_integrator(rx_engine *h, double timestep, double collision_rate, int32_t n_steps,
+                                 const char *splitting) {
+    ENTER(h);
+    int rc = make_move(h, "rx_set_integrator", timestep, collision_rate, n_steps, splitting, 0, &h->move);
+    if (rc) return rc;
     h->have_integrator = true;
     h->state_moves.clear();   // one move for every state again
     return RX_OK;
@@ -250,28 +259,11 @@ extern "C" int rx_set_state_integrator(rx_engine *h, int32_t state, double times
     ENTER(h);
     if (!h->have_integrator) RX_FAIL(h, RX_ERR_INVALID, "rx_set_state_integrator: rx_set_integrator must be called first");
     if (state < 0 || state >= h->cfg.n_states) RX_FAIL(h, RX_ERR_INVALID, "rx_set_state_integrator: state out of range");
-    if (!(timestep > 0) || collision_rate < 0 || n_steps < 0) RX_FAIL(h, RX_ERR_INVALID, "rx_set_state_integrator: bad timestep/collision_rate/n_steps");
-    if (!splitting) RX_FAIL(h, RX_ERR_INVALID, "rx_set_state_integrator: null splitting");
-    const size_t n = strlen(splitting);
-    if (n == 0 || n >= RX_MAX_PROGRAM) RX_FAIL(h, RX_ERR_INVALID, "rx_set_state_integrator: splitting must have 1..31 substeps");
-    bool hasV = false, hasR = false, hasO = false;
-    for (size_t i = 0; i < n; i++) {
-        const char c = splitting[i];
-        if (c == 'V') hasV = true; else if (c == 'R') hasR = true; else if (c == 'O') hasO = true;
-        else RX_FAIL(h, RX_ERR_UNSUPPORTED, "rx_set_state_integrator: only R, V and O substeps are supported");
-    }
-    if (!(hasV && hasR && hasO)) RX_FAIL(h, RX_ERR_INVALID, "rx_set_state_integrator: splitting must contain R, V and O");
-    if (h->state_moves.empty()) {   // start from the common move
-        h->state_moves.resize((size_t)h->cfg.n_states);
-        for (auto &m : h->state_moves) {
-            m.dt = h->dt; m.gamma = h->gamma; m.n_steps = h->n_steps; m.reassign = 0;
-            memcpy(m.program, h->program, sizeof(m.program));
-        }
-    }
-    rx_state_move &m = h->state_moves[(size_t)state];
-    m.dt = timestep; m.gamma = collision_rate; m.n_steps = n_steps; m.reassign = reassign_velocities ? 1 : 0; m.set = true;
-    memset(m.program, 0, sizeof(m.program));
-    memcpy(m.program, splitting, n);
+    rx_state_move m;
+    int rc = make_move(h, "rx_set_state_integrator", timestep, collision_rate, n_steps, splitting, reassign_velocities, &m);
+    if (rc) return rc;
+    if (h->state_moves.empty()) h->state_moves.assign((size_t)h->cfg.n_states, h->move);   // start from the common move
+    h->state_moves[(size_t)state] = m;
     h->state_moves_dirty = true;
     return RX_OK;
 }
@@ -457,19 +449,27 @@ extern "C" int rx_propagate_retry(rx_engine *h, uint64_t seed, uint64_t iteratio
     return finish_propagate(h, T, nan_flags, "rx_propagate_retry");
 }
 
-static int finish_propagate(rx_engine *h, PhaseTimer &T, int32_t *nan_flags, const char *who) {
-    RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream));
-    T.accumulate();
+// The NaN flags of the last propagation: *any tells whether an owned replica has one; nan_flags[K], when given, receives the
+// owned replicas' flags and 0 for the others.
+static int owned_nan_flags(rx_engine *h, int32_t *nan_flags, bool *any) {
     const int K = h->cfg.n_replicas;
     std::vector<int> f(K, 0);
     RX_CHECK_CUDA(h, cudaMemcpy(f.data(), h->d_nan, sizeof(int) * K, cudaMemcpyDeviceToHost));
-    int any = 0;
+    *any = false;
     for (int k = 0; k < K; k++) {
-        const bool mine = k >= h->k0 && k < h->k0 + h->kloc;
-        const int v = mine ? f[k] : 0;
+        const int v = (k >= h->k0 && k < h->k0 + h->kloc) ? f[k] : 0;
         if (nan_flags) nan_flags[k] = v;
-        any |= v;
+        *any |= v != 0;
     }
+    return RX_OK;
+}
+
+static int finish_propagate(rx_engine *h, PhaseTimer &T, int32_t *nan_flags, const char *who) {
+    RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream));
+    T.accumulate();
+    bool any = false;
+    int rc = owned_nan_flags(h, nan_flags, &any);
+    if (rc) return rc;
     if (any) RX_FAIL(h, RX_ERR_NAN, std::string(who) + ": NaN encountered in positions, velocities or potential energy");
     return RX_OK;
 }
@@ -595,20 +595,15 @@ extern "C" int rx_mix_stream_position(rx_engine *h, int32_t stream, uint64_t *wo
     return RX_OK;
 }
 
-extern "C" int rx_run_iterations(rx_engine *h, int32_t n_iterations, int32_t mixing, uint64_t seed,
-                                 uint64_t first_iteration, int32_t reassign) {
-    ENTER(h);
-    int rc = check_ready(h, "rx_run_iterations");
-    if (rc) return rc;
-    if (!h->have_integrator) RX_FAIL(h, RX_ERR_INVALID, "rx_run_iterations: rx_set_integrator must be called first");
-    if (mixing < 0 || mixing > 2) RX_FAIL(h, RX_ERR_INVALID, "rx_run_iterations: mixing must be 0, 1 or 2");
-    const long long K = h->cfg.n_replicas;
+// The fused iteration loop of multistatesampler.py:776-782, n_iterations times: phase 0 on the previous iteration's energies
+// (`step(iteration, &launches)`: a mixing step, a SAMS step or nothing) -> propagate -> energies.  Messages start with `who`.
+template <class Step>
+static int run_iterations(rx_engine *h, const char *who, int32_t n_iterations, uint64_t seed, uint64_t first_iteration,
+                          int32_t reassign, Step &&step) {
     for (int it = 0; it < n_iterations; it++) {
-        // multistatesampler.py:776-782: mix (with the previous iteration's energies) -> propagate -> energies
         int lm = 0, lp = 0, le = 0;
         PhaseTimer Tm(h, 0);
-        if (mixing == 1) rc = rxi_mix_swap_all(h, K * K * K, &lm);
-        else if (mixing == 2) rc = rxi_mix_swap_neighbors(h, &lm);
+        int rc = step(first_iteration + it, &lm);
         if (rc) return rc;
         Tm.stop(lm);
         PhaseTimer Tp(h, 1);
@@ -622,19 +617,30 @@ extern "C" int rx_run_iterations(rx_engine *h, int32_t n_iterations, int32_t mix
         if (rc) return rc;
         Te.stop(le);
         RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream));
-        const double m0 = h->phase_ms[0];
         Tm.accumulate(); Tp.accumulate(); Te.accumulate();
-        if (getenv("RX_TRACE_ITER"))
-            fprintf(stderr, "[iter %d] mix %.2f ms (walker %.2f ms, exact-path lanes %lld, rounds %lld)\n", it, h->phase_ms[0] - m0,
-                    h->mix_stats[4] / 1e3, h->mix_stats[1], h->mix_stats[0]);
     }
-    rc = check_device_error(h);
+    int rc = check_device_error(h);
     if (rc) return rc;
-    std::vector<int> f(K, 0);
-    RX_CHECK_CUDA(h, cudaMemcpy(f.data(), h->d_nan, sizeof(int) * K, cudaMemcpyDeviceToHost));
-    for (int k = h->k0; k < h->k0 + h->kloc; k++)
-        if (f[k]) RX_FAIL(h, RX_ERR_NAN, "rx_run_iterations: NaN encountered in a replica");
+    bool any = false;
+    rc = owned_nan_flags(h, nullptr, &any);
+    if (rc) return rc;
+    if (any) RX_FAIL(h, RX_ERR_NAN, std::string(who) + ": NaN encountered in a replica");
     return RX_OK;
+}
+
+extern "C" int rx_run_iterations(rx_engine *h, int32_t n_iterations, int32_t mixing, uint64_t seed,
+                                 uint64_t first_iteration, int32_t reassign) {
+    ENTER(h);
+    int rc = check_ready(h, "rx_run_iterations");
+    if (rc) return rc;
+    if (!h->have_integrator) RX_FAIL(h, RX_ERR_INVALID, "rx_run_iterations: rx_set_integrator must be called first");
+    if (mixing < 0 || mixing > 2) RX_FAIL(h, RX_ERR_INVALID, "rx_run_iterations: mixing must be 0, 1 or 2");
+    const long long K = h->cfg.n_replicas;
+    return run_iterations(h, "rx_run_iterations", n_iterations, seed, first_iteration, reassign, [&](uint64_t, int *lm) {
+        if (mixing == 1) return rxi_mix_swap_all(h, K * K * K, lm);
+        if (mixing == 2) return rxi_mix_swap_neighbors(h, lm);
+        return (int)RX_OK;
+    });
 }
 
 // ---- SAMS (rx_sams.cuh) ------------------------------------------------------------------------------------------------------
@@ -671,34 +677,10 @@ extern "C" int rx_sams_run_iterations(rx_engine *h, int32_t n_iterations, uint64
     int rc = check_ready(h, "rx_sams_run_iterations");
     if (rc) return rc;
     if (!h->have_integrator) RX_FAIL(h, RX_ERR_INVALID, "rx_sams_run_iterations: rx_set_integrator must be called first");
-    const long long K = h->cfg.n_replicas;
-    for (int it = 0; it < n_iterations; it++) {
-        // multistatesampler.py:776-782 with sams.py:395-437 as the mixing: jump + weight update -> propagate -> energies
-        int lm = 0, lp = 0, le = 0;
-        PhaseTimer Tm(h, 0);
-        rc = rxi_sams_step(h, (long long)(first_iteration + it), first_iteration + it > 0 ? 1 : 0, &lm);
-        if (rc) return rc;
-        Tm.stop(lm);
-        PhaseTimer Tp(h, 1);
-        rc = rxi_propagate(h, seed, first_iteration + it, reassign, &lp);
-        if (rc) return rc;
-        Tp.stop(lp);
-        PhaseTimer Te(h, 2);
-        rc = rxi_compute_energy_rows(h, &le);
-        if (rc) return rc;
-        rc = rxi_allgather_energies(h);
-        if (rc) return rc;
-        Te.stop(le);
-        RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream));
-        Tm.accumulate(); Tp.accumulate(); Te.accumulate();
-    }
-    rc = check_device_error(h);
-    if (rc) return rc;
-    std::vector<int> f(K, 0);
-    RX_CHECK_CUDA(h, cudaMemcpy(f.data(), h->d_nan, sizeof(int) * K, cudaMemcpyDeviceToHost));
-    for (int k = h->k0; k < h->k0 + h->kloc; k++)
-        if (f[k]) RX_FAIL(h, RX_ERR_NAN, "rx_sams_run_iterations: NaN encountered in a replica");
-    return RX_OK;
+    // sams.py:395-437 as the mixing: jump + weight update
+    return run_iterations(h, "rx_sams_run_iterations", n_iterations, seed, first_iteration, reassign, [&](uint64_t iteration, int *lm) {
+        return rxi_sams_step(h, (long long)iteration, iteration > 0 ? 1 : 0, lm);
+    });
 }
 
 extern "C" int rx_get_phase_times(rx_engine *h, double ms[4], int64_t counts[4], int32_t reset) {

@@ -16,6 +16,7 @@ namespace cg = cooperative_groups;
 #include <math.h>
 #include <string.h>
 #include <stdlib.h>
+#include <type_traits>
 
 // ---------------------------------------------------------------------------------------------------
 // Philox4x32-10 counter-based generator: noise is a pure function of (seed, iteration, replica, atom, step)
@@ -55,28 +56,29 @@ __device__ __forceinline__ float fast_rcp(float x) { float y; asm("rcp.approx.ft
 __device__ __forceinline__ float fast_rsqrt(float x) { float y; asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
 // ---------------------------------------------------------------------------------------------------
+// A move as the kernels see it (move_dev()).  A launch carries its move in DynParams::mv; when the states carry different
+// moves (multistatesampler.py:906-910: one MCMCMove per state) a table holds one per state, and a replica is propagated with
+// the move of the state it is in.  (Field order: inside DynParams, dt and n_steps fall on 8-byte boundaries, so the
+// kernels read dt, a and n_steps, n_prog in pairs.)
+struct MoveDev {
+    float dt, a, b;             // timestep, O-step coefficients exp(-gamma h), sqrt(1-exp(-2 gamma h))
+    int reassign;
+    double dt_d, a_d, b_d;      // the same in f64 (the molecule kernel)
+    int n_steps, n_prog, nV, nR, nO;
+    char prog[RX_MAX_PROGRAM];
+};
+
 struct DynParams {
     int N, kind;
     float Lx, Ly, Lz, iLx, iLy, iLz;
     float rc2, rs2, rs, inv_w;  // cutoff^2, switch^2, switch, 1/(rc-rs)
     int use_switch, annihilate, c_is_6;
     float sc_c;                 // softcore_c
-    float dt, a, b;             // timestep, O-step coefficients exp(-gamma h), sqrt(1-exp(-2 gamma h))
-    double dt_d, a_d, b_d;      // the same in f64 (the molecule kernel)
-    int n_steps, n_prog, nV, nR, nO;
+    MoveDev mv;                 // the launch's move
     int maxnb;                  // Verlet-list capacity per atom (0: all-pairs only)
     int sort_atoms;             // re-deal atoms to threads by neighbour count at every list build
     float rl2, rin2;            // (cutoff + skin_out)^2, (cutoff + skin_in)^2
     float half_in2, half_out2;  // (skin_in/2)^2, ((skin_out - skin_in)/2)^2
-    char prog[RX_MAX_PROGRAM];
-};
-
-// One entry per thermodynamic state when the states carry different moves (multistatesampler.py:906-910: one MCMCMove per
-// state); a replica is propagated with the move of the state it is in.
-struct MoveDev {
-    float dt, a, b;
-    int n_steps, n_prog, nV, nR, nO, reassign;
-    char prog[RX_MAX_PROGRAM];
 };
 
 struct PairLam { float la, ob; };
@@ -218,21 +220,22 @@ __device__ __forceinline__ void lj_forces(const DynParams &p, const PairCtx &c, 
 //
 // Positions are double buffered: a force evaluation writes the moved positions into the buffer the previous
 // evaluation did not read, and the displacement vote (__syncthreads_or) is the only barrier of the step.
-// A replica may be split over a cluster of CL thread blocks (CL = 1, 2 or 4; chosen when there are fewer replicas than SMs):
-// block q of the cluster owns the atoms [q Nq, (q+1) Nq), every block keeps ALL positions in its own shared memory -- a block
-// writes the new positions of its atoms into every block's buffer through distributed shared memory -- and the step's only
-// barrier becomes a cluster barrier.  The displacement votes are cluster wide, so the lists are rebuilt at the same steps and
-// with the same contents as in one block: trajectories do not depend on CL (each atom sums its own list in list order, noise
-// is keyed by atom id).
-// PS: per-state moves (the integrator parameters come from `moves[state]` instead of `p`).
-template <bool C6, bool SW, int CL, bool PS = false>
+// A replica may be split over a cluster of CL = 4 thread blocks (prop_plan() chooses it for a few large replicas, CL = 1
+// otherwise): block q of the cluster owns the atoms [q Nq, (q+1) Nq), every block keeps ALL positions in its own shared
+// memory -- a block writes the new positions of its atoms into every block's buffer through distributed shared memory -- and
+// the step's only barrier becomes a cluster barrier.  The displacement votes are cluster wide, so the lists are rebuilt at the
+// same steps and with the same contents as in one block: trajectories do not depend on CL (each atom sums its own list in list
+// order, noise is keyed by atom id).
+// PS: per-state moves (the move comes from `moves[state]` instead of `p.mv`).
+template <bool C6, bool SW, int CL, bool PS>
 __global__ void __launch_bounds__(1024) k_propagate(DynParams p, const float4 *__restrict__ atom,
                                                     const StateDev *__restrict__ states, const int *__restrict__ perm,
                                                     float4 *__restrict__ pos, float4 *__restrict__ vel, int k0,
-                                                    uint2 key, uint32_t iteration, int reassign,
+                                                    uint2 key, uint32_t iteration,
                                                     double *__restrict__ pot, double *__restrict__ kin,
                                                     int *__restrict__ nan_flag, const int *__restrict__ only,
                                                     const MoveDev *__restrict__ moves) {
+    static_assert(CL == 1 || CL == 4, "a replica runs in one block or in a cluster of four");
     extern __shared__ float4 s_dyn[];
     // (the whole cluster takes this exit together: `only` is indexed by replica)
     if (only && !only[k0 + blockIdx.x / CL]) return;   // a retry launch propagates the replicas that failed, nothing else
@@ -265,13 +268,12 @@ __global__ void __launch_bounds__(1024) k_propagate(DynParams p, const float4 *_
     const StateDev st = states[perm[k]];
     const PairLam lam = {(float)st.la, (float)st.ob};
     // the move: the launch's, or the one of this replica's state
-    const MoveDev *mv = PS ? moves + perm[k] : nullptr;
-    const float m_dt = PS ? mv->dt : p.dt, m_a = PS ? mv->a : p.a, m_b = PS ? mv->b : p.b;
-    const int m_steps = PS ? mv->n_steps : p.n_steps, m_nprog = PS ? mv->n_prog : p.n_prog, m_nV = PS ? mv->nV : p.nV,
-              m_nR = PS ? mv->nR : p.nR;
+    const MoveDev &mv = PS ? moves[perm[k]] : p.mv;
+    // (read once: loaded from `moves` inside the step loop, they cost the per-state variants a register spill)
+    const float m_a = mv.a, m_b = mv.b;
+    const int m_steps = mv.n_steps, m_nprog = mv.n_prog;
     // (the program is interpreted: the compiler does not hoist these divisions out of the step loop; same values, same bits)
-    const float h_V = m_dt / (float)m_nV, h_R = m_dt / (float)m_nR;
-    if (PS) reassign = mv->reassign;
+    const float h_V = mv.dt / (float)mv.nV, h_R = mv.dt / (float)mv.nR;
     float sig_i, se_i, inv_m, sigma_v;
     bool alch_i;
     auto load_atom = [&]() {
@@ -283,7 +285,7 @@ __global__ void __launch_bounds__(1024) k_propagate(DynParams p, const float4 *_
     float4 x4 = active ? pos[(size_t)r * p.N + a] : make_float4(0, 0, 0, 0);
     float4 v4 = active ? vel[(size_t)r * p.N + a] : make_float4(0, 0, 0, 0);
     float x = x4.x, y = x4.y, z = x4.z, vx = v4.x, vy = v4.y, vz = v4.z;
-    if (reassign && active) {  // context.setVelocitiesToTemperature, mcmc.py:711
+    if (mv.reassign && active) {  // context.setVelocitiesToTemperature, mcmc.py:711
         const float3 g = philox_normal3(philox4x32_10(make_uint4(a, 0x80000000u, k, iteration), key));
         vx = sigma_v * g.x; vy = sigma_v * g.y; vz = sigma_v * g.z;
     }
@@ -446,7 +448,7 @@ __global__ void __launch_bounds__(1024) k_propagate(DynParams p, const float4 *_
     float dummy;
     for (int s = 0; s < m_steps; s++) {
         for (int q = 0; q < m_nprog; q++) {
-            const char op = PS ? mv->prog[q] : p.prog[q];
+            const char op = mv.prog[q];
             if (op == 'V') {
                 if (!f_valid) { compute_forces(false, dummy); f_valid = true; }
                 const float h = h_V;
@@ -711,7 +713,22 @@ int rxi_convert_out(rx_engine *h, const float4 *src, int first_local, int count,
 #include "rx_molecule.cuh"
 
 // ---------------------------------------------------------------------------------------------------
-static int fill_dyn(rx_engine *h, DynParams &p) {
+// The kernels' form of a move.
+static MoveDev move_dev(const rx_state_move &m) {
+    MoveDev d;
+    memset(&d, 0, sizeof(d));
+    for (const char *q = m.program; *q; q++) {
+        if (*q == 'V') d.nV++; else if (*q == 'R') d.nR++; else d.nO++;
+        d.prog[d.n_prog++] = *q;
+    }
+    d.dt = (float)m.dt; d.n_steps = m.n_steps; d.reassign = m.reassign;
+    const double hO = m.dt / (d.nO > 0 ? d.nO : 1);   // integrators.py:1141-1146
+    d.dt_d = m.dt; d.a_d = exp(-m.gamma * hO); d.b_d = sqrt(1.0 - exp(-2.0 * m.gamma * hO));
+    d.a = (float)d.a_d; d.b = (float)d.b_d;
+    return d;
+}
+
+static void fill_dyn(const rx_engine *h, DynParams &p) {
     const rx_config &c = h->cfg;
     memset(&p, 0, sizeof(p));
     p.N = c.n_atoms; p.kind = c.system_kind;
@@ -721,16 +738,7 @@ static int fill_dyn(rx_engine *h, DynParams &p) {
     p.inv_w = (float)(1.0 / (c.r_cutoff - c.r_switch));
     p.use_switch = c.use_switch; p.annihilate = c.annihilate_sterics;
     p.c_is_6 = (c.softcore_c == 6.0); p.sc_c = (float)c.softcore_c;
-    p.dt = (float)h->dt; p.n_steps = h->n_steps;
-    int nV = 0, nR = 0, nO = 0, n = 0;
-    for (const char *q = h->program; *q; q++, n++) { if (*q == 'V') nV++; else if (*q == 'R') nR++; else nO++; p.prog[n] = *q; }
-    p.n_prog = n; p.nV = nV; p.nR = nR; p.nO = nO;
-    p.maxnb = 0; p.sort_atoms = 0; p.rl2 = p.rin2 = p.rc2; p.half_in2 = p.half_out2 = 0.f;
-    const double hO = h->dt / (nO > 0 ? nO : 1);   // integrators.py:1141-1146
-    p.a = (float)exp(-h->gamma * hO);
-    p.b = (float)sqrt(1.0 - exp(-2.0 * h->gamma * hO));
-    p.dt_d = h->dt; p.a_d = exp(-h->gamma * hO); p.b_d = sqrt(1.0 - exp(-2.0 * h->gamma * hO));
-    return RX_OK;
+    p.mv = move_dev(h->move);
 }
 
 // The per-state move table (rx_set_state_integrator), uploaded when it changed.
@@ -738,22 +746,98 @@ int rxi_upload_state_moves(rx_engine *h) {
     if (!h->state_moves_dirty) return RX_OK;
     const int M = h->cfg.n_states;
     std::vector<MoveDev> tab((size_t)M);
-    for (int l = 0; l < M; l++) {
-        const rx_state_move &m = h->state_moves[(size_t)l];
-        MoveDev &d = tab[(size_t)l];
-        memset(&d, 0, sizeof(d));
-        int n = 0, nV = 0, nR = 0, nO = 0;
-        for (const char *q = m.program; *q; q++, n++) { if (*q == 'V') nV++; else if (*q == 'R') nR++; else nO++; d.prog[n] = *q; }
-        d.n_prog = n; d.nV = nV; d.nR = nR; d.nO = nO;
-        d.dt = (float)m.dt; d.n_steps = m.n_steps; d.reassign = m.reassign;
-        const double hO = m.dt / (nO > 0 ? nO : 1);   // integrators.py:1141-1146
-        d.a = (float)exp(-m.gamma * hO);
-        d.b = (float)sqrt(1.0 - exp(-2.0 * m.gamma * hO));
-    }
+    for (int l = 0; l < M; l++) tab[(size_t)l] = move_dev(h->state_moves[(size_t)l]);
     if (!h->d_moves) RX_CHECK_CUDA(h, cudaMalloc(&h->d_moves, sizeof(MoveDev) * (size_t)M));
     RX_CHECK_CUDA(h, cudaMemcpyAsync(h->d_moves, tab.data(), sizeof(MoveDev) * (size_t)M, cudaMemcpyHostToDevice, h->stream));
     RX_CHECK_CUDA(h, cudaStreamSynchronize(h->stream));   // (tab is a stack object)
     h->state_moves_dirty = false;
+    return RX_OK;
+}
+
+// How k_propagate runs for a particle system: the launch shape and the neighbour-list geometry of DynParams.
+struct PropPlan {
+    int cl;          // blocks per replica (one thread-block cluster): 1 or 4
+    int threads;     // per block: one thread per atom of the block, whole warps
+    size_t smem;     // dynamic shared memory per block
+    int maxnb, sort_atoms;
+    float rl2, rin2, half_in2, half_out2;
+};
+
+static PropPlan prop_plan(const rx_engine *h) {
+    const rx_config &c = h->cfg;
+    const int N = c.n_atoms;
+    const bool lj = c.system_kind == RX_SYSTEM_LJ_ALCH;
+    PropPlan pl = {};
+    // Measured on the 512-atom fluid (500 steps, in the iteration loop, profiles/r2_cluster_propagate.txt): 32 replicas
+    // 2.27-2.36 ms in one block, 2.20-2.29 in a cluster of four; 64 replicas 2.28-2.37 / 2.31-2.39.  A block of 128 threads
+    // leaves ONE warp per scheduler, which runs the step's ~1100 dependent instructions no faster than four warps sharing a
+    // scheduler do: the split only pays for the few replicas that would otherwise leave three quarters of the GPU idle, so
+    // that is the only case it is chosen for.  Per-state moves have no cluster variant.
+    pl.cl = (lj && N >= 256 && h->kloc * 4 <= h->n_sms && h->state_moves.empty()) ? 4 : 1;
+    pl.threads = ((N + pl.cl - 1) / pl.cl + 31) / 32 * 32;
+    pl.rl2 = pl.rin2 = (float)(c.r_cutoff * c.r_cutoff);
+    // shared memory: two position buffers + the parameter records + per-thread reference positions + the list area
+    const size_t atoms_bytes = (size_t)3 * RX_MAX_ATOMS * sizeof(float4) + (size_t)pl.threads * sizeof(float4);
+    size_t area = (size_t)pl.threads * sizeof(double2);  // the list area doubles as scratch for the final reductions
+    if (lj && N >= 64 && !getenv("RX_NO_VERLET")) {
+        // Dual neighbour list: outer skin 0.40 nm (at 300 K and 10/ps friction the all-pairs build usually lasts a
+        // whole 500-step launch), inner skin 0.05 nm (a re-partition of the column about every 25 steps; both tuned
+        // on the 512-atom fluid, see profiles/prop_r1_v6.summary.txt).  Capacity from the
+        // shared-memory budget (two CTAs per SM up to 512 atoms); denser systems fall back to all-pairs in the kernel.
+        double skin_in = 0.05;
+        double rl = c.r_cutoff + 0.40;
+        for (int d = 0; d < 3; d++) if (rl > 0.5 * c.box[d]) rl = 0.5 * c.box[d];
+        const double eff_out = rl - c.r_cutoff;
+        if (skin_in > eff_out / 3.0) skin_in = eff_out / 3.0;
+        if (eff_out > 0.03) {
+            const size_t budget = (pl.threads > 512 ? 200 : 112) * 1024;
+            int cap = (int)((budget - atoms_bytes) / ((size_t)pl.threads * sizeof(unsigned short)));
+            if (cap > 128) cap = 128;
+            if (cap >= 8) {
+                pl.maxnb = cap;
+                pl.rl2 = (float)(rl * rl);
+                pl.rin2 = (float)((c.r_cutoff + skin_in) * (c.r_cutoff + skin_in));
+                pl.half_in2 = (float)(0.25 * skin_in * skin_in);
+                pl.half_out2 = (float)(0.25 * (eff_out - skin_in) * (eff_out - skin_in));
+                const size_t list_bytes = (((size_t)cap * pl.threads * sizeof(unsigned short)) + 15) / 16 * 16;
+                // scratch of the atom re-assignment: velocities, order, per-warp bin counts, bin bases
+                const size_t sort_bytes = (size_t)pl.threads * (sizeof(float4) + 2) + (size_t)(pl.threads / 32 + 1) * RX_SORT_BINS * 2;
+                pl.sort_atoms = list_bytes >= sort_bytes ? 1 : 0;
+                if (list_bytes > area) area = list_bytes;
+            }
+        }
+    }
+    pl.smem = atoms_bytes + area;
+    return pl;
+}
+
+// Calls f(C6, SW) -- std::integral_constant<bool, ...> arguments -- with the pair-function specialisation of the engine.
+template <class F>
+static int with_pair_kind(const DynParams &p, F &&f) {
+    using T = std::true_type;
+    using U = std::false_type;
+    if (p.c_is_6) return p.use_switch ? f(T(), T()) : f(T(), U());
+    return p.use_switch ? f(U(), T()) : f(U(), U());
+}
+
+template <bool C6, bool SW, int CL, bool PS>
+static int launch_propagate(rx_engine *h, const PropPlan &pl, const DynParams &p, uint2 key, uint32_t iteration,
+                            const int *d_only) {
+    cudaLaunchConfig_t lc = {};
+    lc.gridDim = dim3((unsigned)(h->kloc * CL));
+    lc.blockDim = dim3((unsigned)pl.threads);
+    lc.dynamicSmemBytes = pl.smem;
+    lc.stream = h->stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = (unsigned)CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    lc.attrs = at;
+    lc.numAttrs = 1;
+    if (pl.smem > 48 * 1024)
+        RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_propagate<C6, SW, CL, PS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+    RX_CHECK_CUDA(h, cudaLaunchKernelEx(&lc, k_propagate<C6, SW, CL, PS>, p, (const float4 *)h->d_atom, (const StateDev *)h->d_states,
+                                        (const int *)h->d_perm, h->d_pos, h->d_vel, h->k0, key, iteration, h->d_pot, h->d_kin,
+                                        h->d_nan, d_only, (const MoveDev *)h->d_moves));
     return RX_OK;
 }
 
@@ -762,104 +846,35 @@ int rxi_propagate(rx_engine *h, uint64_t seed, uint64_t iteration, int reassign,
     DynParams p;
     fill_dyn(h, p);
     const int N = h->cfg.n_atoms;
+    const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32) ^ (uint32_t)(iteration >> 32));
     if (h->cfg.system_kind == RX_SYSTEM_MOLECULE) {
         if (!h->state_moves.empty()) RX_FAIL(h, RX_ERR_UNSUPPORTED, "rx_propagate: per-state moves are not provided for molecules");
-        const uint2 mkey = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32) ^ (uint32_t)(iteration >> 32));
         const MolDev *md = (const MolDev *)h->mol_dev;
         const bool no_star = getenv("RX_MOL_NO_STAR") != nullptr;   // cross-check: the general cluster path for every molecule
         auto kern = (md->max_cluster <= 3 && !no_star) ? k_propagate_mol<true> : k_propagate_mol<false>;
         kern<<<h->kloc, 32 * MOL_WARPS, md->dyn_shared_bytes, h->stream>>>(*md, p, (const StateDev *)h->d_states, (const int *)h->d_perm, (double *)h->d_pos,
-                                                                           (double *)h->d_vel, h->k0, mkey, (uint32_t)iteration, reassign, h->d_pot,
+                                                                           (double *)h->d_vel, h->k0, key, (uint32_t)iteration, reassign, h->d_pot,
                                                                            h->d_kin, h->d_nan, d_only);
         RX_CHECK_CUDA(h, cudaGetLastError());
         (*launches)++;
         return RX_OK;
     }
     if (N > 1024) RX_FAIL(h, RX_ERR_UNSUPPORTED, "rx_propagate: more than 1024 atoms per replica is not supported yet");
-    // Blocks per replica (a thread-block cluster; RX_CLUSTER = 1 | 2 | 4 overrides).  Measured on the 512-atom fluid (500
-    // steps, in the iteration loop): 32 replicas 2.27-2.36 ms in one block, 2.30-2.59 in two, 2.20-2.29 in four; 64 replicas
-    // 2.28-2.37 / 2.31-2.41 / 2.31-2.39.  A block of 128 threads leaves ONE warp per scheduler, which runs the step's
-    // ~1100 dependent instructions no faster than four warps sharing a scheduler do: the split only pays for the few
-    // replicas that would otherwise leave three quarters of the GPU idle, so that is the only case it is chosen for.
-    int cl = 1;
-    if (h->cfg.system_kind == RX_SYSTEM_LJ_ALCH && N >= 256) {
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->cfg.device);
-        if (h->kloc * 4 <= sms) cl = 4;
-        if (const char *e = getenv("RX_CLUSTER")) { const int v = atoi(e); if (v == 1 || v == 2 || v == 4) cl = v; }
-    }
     const bool per_state = !h->state_moves.empty();
-    if (per_state) {
-        cl = 1;
-        int rcm = rxi_upload_state_moves(h);
-        if (rcm) return rcm;
-    }
-    const int n_per = (N + cl - 1) / cl;
-    const int threads = ((n_per + 31) / 32) * 32;
-    // shared memory: two position buffers + the parameter records + per-thread reference positions + the list area
-    const size_t atoms_bytes = (size_t)3 * RX_MAX_ATOMS * sizeof(float4) + (size_t)threads * sizeof(float4);
-    size_t area = (size_t)threads * sizeof(double2);  // the list area doubles as scratch for the final reductions
-    if (h->cfg.system_kind == RX_SYSTEM_LJ_ALCH && N >= 64 && !getenv("RX_NO_VERLET")) {
-        // Dual neighbour list: outer skin 0.40 nm (at 300 K and 10/ps friction the all-pairs build usually lasts a
-        // whole 500-step launch), inner skin 0.05 nm (a re-partition of the column about every 25 steps; both tuned
-        // on the 512-atom fluid, see profiles/prop_r1_v6.summary.txt).  Capacity from the
-        // shared-memory budget (two CTAs per SM up to 512 atoms); denser systems fall back to all-pairs in the kernel.
-        const char *so = getenv("RX_SKIN"), *si = getenv("RX_SKIN_IN");
-        const double skin_out = so ? atof(so) : 0.40;
-        double skin_in = si ? atof(si) : 0.05;
-        double rl = h->cfg.r_cutoff + skin_out;
-        for (int d = 0; d < 3; d++) if (rl > 0.5 * h->cfg.box[d]) rl = 0.5 * h->cfg.box[d];
-        const double eff_out = rl - h->cfg.r_cutoff;
-        if (skin_in > eff_out / 3.0) skin_in = eff_out / 3.0;
-        if (eff_out > 0.03) {
-            const size_t budget = (threads > 512 ? 200 : 112) * 1024;
-            int cap = (int)((budget - atoms_bytes) / ((size_t)threads * sizeof(unsigned short)));
-            if (cap > 128) cap = 128;
-            if (cap >= 8) {
-                p.maxnb = cap;
-                p.rl2 = (float)(rl * rl);
-                p.rin2 = (float)((h->cfg.r_cutoff + skin_in) * (h->cfg.r_cutoff + skin_in));
-                p.half_in2 = (float)(0.25 * skin_in * skin_in);
-                p.half_out2 = (float)(0.25 * (eff_out - skin_in) * (eff_out - skin_in));
-                const size_t list_bytes = (((size_t)cap * threads * sizeof(unsigned short)) + 15) / 16 * 16;
-                // scratch of the atom re-assignment: velocities, order, per-warp bin counts, bin bases
-                const size_t sort_bytes = (size_t)threads * (sizeof(float4) + 2) + (size_t)(threads / 32 + 1) * RX_SORT_BINS * 2;
-                p.sort_atoms = (list_bytes >= sort_bytes && !getenv("RX_NO_SORT")) ? 1 : 0;
-                if (list_bytes > area) area = list_bytes;
-            }
-        }
-    }
-    const size_t smem = atoms_bytes + area;
-    const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32) ^ (uint32_t)(iteration >> 32));
-    cudaLaunchConfig_t lc = {};
-    lc.gridDim = dim3((unsigned)(h->kloc * cl));
-    lc.blockDim = dim3((unsigned)threads);
-    lc.dynamicSmemBytes = smem;
-    lc.stream = h->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = (unsigned)cl; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    lc.attrs = at;
-    lc.numAttrs = 1;
+    int rc = per_state ? rxi_upload_state_moves(h) : RX_OK;
+    if (rc) return rc;
+    const PropPlan pl = prop_plan(h);
+    p.maxnb = pl.maxnb; p.sort_atoms = pl.sort_atoms;
+    p.rl2 = pl.rl2; p.rin2 = pl.rin2; p.half_in2 = pl.half_in2; p.half_out2 = pl.half_out2;
+    p.mv.reassign = reassign;
     const uint32_t it32 = (uint32_t)iteration;
-#define RX_LAUNCH_PROPAGATE(C6, SW, CL, PS)                                                                               \
-    do {                                                                                                                   \
-        if (smem > 48 * 1024)                                                                                              \
-            RX_CHECK_CUDA(h, cudaFuncSetAttribute(k_propagate<C6, SW, CL, PS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        RX_CHECK_CUDA(h, cudaLaunchKernelEx(&lc, k_propagate<C6, SW, CL, PS>, p, (const float4 *)h->d_atom, (const StateDev *)h->d_states, \
-                                            (const int *)h->d_perm, h->d_pos, h->d_vel, h->k0, key, it32, reassign, h->d_pot, \
-                                            h->d_kin, h->d_nan, d_only, (const MoveDev *)h->d_moves));                    \
-    } while (0)
-#define RX_LAUNCH_PROPAGATE_CL(C6, SW)                                                                                    \
-    do {                                                                                                                   \
-        if (per_state) RX_LAUNCH_PROPAGATE(C6, SW, 1, true);                                                               \
-        else if (cl == 4) RX_LAUNCH_PROPAGATE(C6, SW, 4, false); else if (cl == 2) RX_LAUNCH_PROPAGATE(C6, SW, 2, false); \
-        else RX_LAUNCH_PROPAGATE(C6, SW, 1, false);                                                                        \
-    } while (0)
-    if (p.c_is_6) { if (p.use_switch) RX_LAUNCH_PROPAGATE_CL(true, true); else RX_LAUNCH_PROPAGATE_CL(true, false); }
-    else { if (p.use_switch) RX_LAUNCH_PROPAGATE_CL(false, true); else RX_LAUNCH_PROPAGATE_CL(false, false); }
-#undef RX_LAUNCH_PROPAGATE_CL
-#undef RX_LAUNCH_PROPAGATE
+    rc = with_pair_kind(p, [&](auto c6, auto sw) -> int {
+        constexpr bool C6 = decltype(c6)::value, SW = decltype(sw)::value;
+        if (per_state) return launch_propagate<C6, SW, 1, true>(h, pl, p, key, it32, d_only);
+        if (pl.cl == 4) return launch_propagate<C6, SW, 4, false>(h, pl, p, key, it32, d_only);
+        return launch_propagate<C6, SW, 1, false>(h, pl, p, key, it32, d_only);
+    });
+    if (rc) return rc;
     RX_CHECK_CUDA(h, cudaGetLastError());
     (*launches)++;
     return RX_OK;
@@ -1007,14 +1022,12 @@ int rxi_minimize(rx_engine *h, double tolerance, int max_iterations, double *d_r
     if (N > 1024) RX_FAIL(h, RX_ERR_UNSUPPORTED, "rx_minimize: more than 1024 atoms per replica is not supported yet");
     const int threads = ((N + 31) / 32) * 32;
     const size_t smem = (size_t)2 * RX_MAX_ATOMS * sizeof(float4);
-#define RX_LAUNCH_MINIMIZE(C6, SW)                                                                                         \
-    k_minimize<C6, SW><<<h->kloc, threads, smem, h->stream>>>(p, h->d_atom, h->d_states, h->d_perm, h->d_pos, h->k0,       \
-                                                              (float)tolerance, max_iterations, d_rms, d_iters)
-    if (p.c_is_6) { if (p.use_switch) RX_LAUNCH_MINIMIZE(true, true); else RX_LAUNCH_MINIMIZE(true, false); }
-    else { if (p.use_switch) RX_LAUNCH_MINIMIZE(false, true); else RX_LAUNCH_MINIMIZE(false, false); }
-#undef RX_LAUNCH_MINIMIZE
-    RX_CHECK_CUDA(h, cudaGetLastError());
-    return RX_OK;
+    return with_pair_kind(p, [&](auto c6, auto sw) -> int {
+        k_minimize<decltype(c6)::value, decltype(sw)::value><<<h->kloc, threads, smem, h->stream>>>(
+            p, h->d_atom, h->d_states, h->d_perm, h->d_pos, h->k0, (float)tolerance, max_iterations, d_rms, d_iters);
+        RX_CHECK_CUDA(h, cudaGetLastError());
+        return RX_OK;
+    });
 }
 
 int rxi_randomize_velocities(rx_engine *h, uint64_t seed, uint64_t stream_id) {

@@ -49,16 +49,17 @@ struct MixCtl {          // device-resident control block of the resumable mixin
     long long aux;       // k_mix_walk2c: candidate index reached (extent of its sparse commit log)
 };
 
+// One Langevin move: timestep, friction, steps per launch, splitting program and velocity reassignment.
 struct rx_state_move {
     double dt = 0, gamma = 0;
     int n_steps = 0, reassign = 0;
     char program[RX_MAX_PROGRAM] = {0};
-    bool set = false;
 };
 
 struct rx_engine {
     rx_config cfg;
     int k0 = 0, kloc = 0;  // owned replicas [k0, k0+kloc)
+    int n_sms = 0;         // streaming multiprocessors of cfg.device
     cudaStream_t stream = nullptr, stream_rng = nullptr;
     cudaEvent_t ev[8] = {};
     cudaEvent_t ev_user[2] = {};
@@ -89,10 +90,7 @@ struct rx_engine {
     // energy kernel scratch: lambda-controlled pairs per owned replica
     double4 *d_pairs = nullptr;  // (r, sigma, eps, S) ... see rx_dynamics.cu
     int pair_cap = 0;
-    // integrator
-    double dt = 0, gamma = 0;
-    int n_steps = 0;
-    char program[RX_MAX_PROGRAM] = {0};
+    rx_state_move move;                      // the move of every state (rx_set_integrator; its reassign is unused)
     void *mol_dev = nullptr;                 // MolDev (host copy of the device table of a RX_SYSTEM_MOLECULE engine)
     std::vector<void *> mol_allocs;
     std::vector<rx_state_move> state_moves;   // per-state moves (empty: one move for all states)

@@ -659,19 +659,19 @@ __global__ void __launch_bounds__(32 * MOL_WARPS) k_propagate_mol(MolDev m, DynP
     __syncwarp();
     const double inv_mass = 1.0 / mass;
     // (the program is interpreted, so the compiler does not hoist these out of the step loop: two f64 divisions per R)
-    const double hm = (double)p.dt_d / p.nV * inv_mass, h = (double)p.dt_d / p.nR, inv_h = 1.0 / h;
+    const double hm = (double)p.mv.dt_d / p.mv.nV * inv_mass, h = (double)p.mv.dt_d / p.mv.nR, inv_h = 1.0 / h;
     double f[3] = {0, 0, 0};
     bool f_valid = false;
     uint32_t ocount = 0;
-    for (int s = 0; s < p.n_steps; s++) {
+    for (int s = 0; s < p.mv.n_steps; s++) {
         if (m.remove_cm) {
             double px = mol_warp_sum(active ? mass * V[a][0] : 0.0), py = mol_warp_sum(active ? mass * V[a][1] : 0.0),
                    pz = mol_warp_sum(active ? mass * V[a][2] : 0.0);
             if (active) { V[a][0] -= px * inv_mt; V[a][1] -= py * inv_mt; V[a][2] -= pz * inv_mt; }
             __syncwarp();
         }
-        for (int q = 0; q < p.n_prog; q++) {
-            const char op = p.prog[q];
+        for (int q = 0; q < p.mv.n_prog; q++) {
+            const char op = p.mv.prog[q];
             if (op == 'V') {
                 if (!f_valid) {
                     __syncthreads();   // warp 0's positions are in shared memory
@@ -705,9 +705,9 @@ __global__ void __launch_bounds__(32 * MOL_WARPS) k_propagate_mol(MolDev m, DynP
             } else {   // 'O'
                 if (active) {
                     const float3 g = philox_normal3(philox4x32_10(make_uint4(a, ocount, k, iteration), key));
-                    V[a][0] = p.a_d * V[a][0] + p.b_d * sg * (double)g.x;
-                    V[a][1] = p.a_d * V[a][1] + p.b_d * sg * (double)g.y;
-                    V[a][2] = p.a_d * V[a][2] + p.b_d * sg * (double)g.z;
+                    V[a][0] = p.mv.a_d * V[a][0] + p.mv.b_d * sg * (double)g.x;
+                    V[a][1] = p.mv.a_d * V[a][1] + p.mv.b_d * sg * (double)g.y;
+                    V[a][2] = p.mv.a_d * V[a][2] + p.mv.b_d * sg * (double)g.z;
                 }
                 ocount++;
                 __syncwarp();

@@ -190,29 +190,51 @@ def test_pair_kernel_variants_match_oracle(use_switch, annihilate, alpha, a, b, 
     e.close()
 
 
-@pytest.mark.parametrize('cl', [2, 4])
-def test_cluster_split_replica_reproduces_single_block_trajectory(monkeypatch, cl):
-    """A replica split over a thread-block cluster (atoms partitioned over 2 or 4 blocks, positions exchanged through
+def test_cluster_split_replica_reproduces_single_block_trajectory():
+    """A replica split over a thread-block cluster (atoms partitioned over 4 blocks, positions exchanged through
     distributed shared memory, cluster-wide displacement votes) must give the SAME trajectory as one block per replica:
     lists are rebuilt at the same steps with the same contents, every atom sums its own list in list order, noise is
-    keyed by atom id.  200 hot steps cross several re-partitions and at least one outer rebuild."""
+    keyed by atom id.  Engine A (3 replicas) runs in clusters of four; engine B has too many replicas for that and runs
+    one block per replica, its first 3 replicas starting where A's do.  200 hot steps cross several re-partitions and
+    at least one outer rebuild."""
+    import torch
     N, K = 512, 3
     s = lj_setup(N=N, n_alch=10, seed=51)
     lambdas = np.array([1.0, 0.5, 0.0]); temps = np.array([500.0, 500.0, 500.0])
     rng = np.random.default_rng(15)
-    v0 = rng.normal(scale=0.3, size=(K, N, 3)).astype(np.float32).astype(np.float64)
+    n_b = torch.cuda.get_device_properties(0).multi_processor_count // 4 + 1
+    v0 = rng.normal(scale=0.3, size=(n_b, N, 3)).astype(np.float32).astype(np.float64)
     out = []
-    for c in (1, cl):
-        monkeypatch.setenv('RX_CLUSTER', str(c))
-        e = make_engine(s, K, K, lambdas, temps, 0.002, 1.0, 200, 'V R O R V')
-        e.set_positions(np.stack([s['x']] * K)); e.set_velocities(v0)
-        e.set_replica_states(np.array([1, 2, 0]))
+    for n in (K, n_b):
+        e = make_engine(s, n, K, lambdas, temps, 0.002, 1.0, 200, 'V R O R V')
+        e.set_positions(np.stack([s['x']] * n)); e.set_velocities(v0[:n])
+        e.set_replica_states(np.array([1, 2, 0] + [k % K for k in range(K, n)]))
         e.propagate(1234, 9)
-        out.append((e.get_positions(), e.get_velocities(), e.get_replica_energies()))
+        x, v, (pe, ke) = e.get_positions(), e.get_velocities(), e.get_replica_energies()
+        out.append((x[:K], v[:K], (pe[:K], ke[:K])))
         e.close()
     (xa, va, (pa, ka)), (xb, vb, (pb, kb)) = out
     assert np.array_equal(xa, xb) and np.array_equal(va, vb)
     assert np.allclose(pa, pb, rtol=1e-12, atol=1e-9) and np.allclose(ka, kb, rtol=1e-12, atol=1e-9)   # other summation order
+
+
+@pytest.mark.parametrize('splitting,code', [('', 'INVALID'), ('VR', 'INVALID'), ('VRXO', 'UNSUPPORTED'),
+                                             ('VRO' * 10 + 'VR', 'INVALID')])
+def test_bad_splitting_is_refused_alike_for_one_move_and_per_state_moves(splitting, code):
+    """rx_set_integrator and rx_set_state_integrator check a splitting with the same rules: empty, without O, with an
+    unknown substep, 32 substeps."""
+    from openmmtools_b200 import _lib
+    from openmmtools_b200._engine import EngineError
+    e = gpu_engine(2, 2, 2, 1)
+    e.set_integrator(0.001, 1.0, 10, 'V R O R V')
+    with pytest.raises(EngineError) as one:
+        e.set_integrator(0.001, 1.0, 10, splitting)
+    with pytest.raises(EngineError) as per_state:
+        e.set_state_integrator(0, 0.001, 1.0, 10, splitting)
+    assert one.value.code == per_state.value.code == getattr(_lib, 'RX_ERR_' + code)
+    assert one.value.message.startswith('rx_set_integrator:')
+    assert per_state.value.message.startswith('rx_set_state_integrator:')
+    e.close()
 
 
 def test_per_state_moves_propagate_each_replica_with_the_move_of_its_state():
